@@ -108,6 +108,23 @@ def make_inputs(wl, seed, jitter=0.0):
     return feats, proj, dv
 
 
+def dump_outputs(outs, directory):
+    """--dump-outputs: writes {name: tensor} as DIR/<name>.npy in float32.  The final maps are written whole up to
+    3 Mi values (one DTU or T&T depth map per GPU), every other array up to 512 Ki values; a larger array is written as a
+    fixed, seeded sample of that many values (flattened) under <name>_sample.npy.  At most 2 x 12 + 12 x 2 = 48 MB."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    for name, t in outs.items():
+        cap = (3 << 20) if name in ("refined_depth", "photometric_confidence") else (1 << 19)
+        v = t.detach().float()
+        if v.numel() > cap:
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            v = v.reshape(-1)[idx.to(v.device)]
+            name += "_sample"
+        np.save(os.path.join(directory, name + ".npy"), v.cpu().numpy().astype(np.float32))
+
+
 def make_net(seed=7):
     import torch
     from mvsformerplusplus_b200 import synth
@@ -223,6 +240,7 @@ def run_ours(a, wl, rank, world, local_rank):
     lane_bufs = [local_buf] + [torch.empty_like(local_buf) for _ in range(n_lanes - 1)]
     lane_gathered = [torch.cuda.Event() for _ in range(n_lanes)]
     step_no = [0]
+    last_outs = [None] * len(dev_inputs)   # --dump-outputs: what the latest step's forward calls returned
 
     def step_resident():
         k = step_no[0] % n_lanes
@@ -234,6 +252,8 @@ def run_ours(a, wl, rank, world, local_rank):
                 out = net.forward_features(f, p, d, TMP)
                 buf[b, 0].copy_(out["refined_depth"][0])
                 buf[b, 1].copy_(out["photometric_confidence"][0])
+                if a.dump_outputs:
+                    last_outs[b] = out
         # the only collective on the path: gather of the depth / confidence maps in item order (SURVEY.md 8e), issued on the
         # main stream in step order on every rank (after the lane's kernels; the other lane keeps running)
         if world > 1:
@@ -291,6 +311,13 @@ def run_ours(a, wl, rank, world, local_rank):
     ms_step = timed(step_resident, a.steps, max(a.warmup, 3))
     launches = _lib.launch_count(reset=True) // (a.steps + max(a.warmup, 3))
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs and rank == 0:   # rank 0's reference views, in item order
+        outs = {k: torch.stack([o[k][0] for o in last_outs]) for k in ("refined_depth", "photometric_confidence")}
+        for s in range(1, 5):
+            for k in ("depth", "photometric_confidence", "prob_volume"):
+                outs[f"stage{s}_{k}"] = torch.stack([o[f"stage{s}"][k][0] for o in last_outs])
+        dump_outputs(outs, a.dump_outputs)
+    last_outs[:] = [None] * len(last_outs)   # released before the end-to-end timing
     ms_e2e = timed(step_e2e, a.steps, max(a.warmup, 3))
     d2h = host_out.numel() * 4
 
@@ -432,7 +459,7 @@ def run_dsweep(a):
         _lib.check(L.mvsf_vis_cnn(P(ent), P(wts), P(vis), V - 1, H, W, st()), "vis_cnn")
         pass_b()
         torch.cuda.synchronize()
-        reps = max(1, a.steps // 3)
+        reps = a.steps
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
         ta = tb = 0.0
         for _ in range(reps):
@@ -450,7 +477,7 @@ def run_dsweep(a):
             "config": {"workload": "dsweep: plane-sweep hypotheses uniform in inverse depth over 425..931 mm, two-gather plan "
                                    "(pass A entropy + pass B aggregation), inputs larger than L2 (283 MB of features)"},
             "roofline": {"bound": "hbm", "peak": peak, "unit": "GB/s", "achieved": best, "frac": best / peak, "traffic": None},
-            "sweep": rows, "gpu_launches": 2 * len(rows) * max(1, a.steps // 3)}
+            "sweep": rows, "gpu_launches": 2 * len(rows) * a.steps}
     print(json.dumps(line), flush=True)
 
 
@@ -467,7 +494,15 @@ def main():
                          "flight measured +8.7 %% (79.8 maps/s) but the attention kernel deadlocks once in a few hundred launches when "
                          "kernels of another stream run next to it (DESIGN.md 5); the bounded waits turn that into a CUDA error")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (final depth and confidence maps, "
+                         "per-stage depth, confidence and probability volume of rank 0's reference views) as DIR/<name>.npy; "
+                         "inputs and weights are seeded, so two builds run with the same arguments can be compared")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.workload == "dsweep"):
+        ap.error("--dump-outputs needs --impl ours and a depth-map workload")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -477,9 +512,7 @@ def main():
         return
     wl = WORKLOADS[a.workload]
     if a.impl == "reference":
-        if a.steps > 3:
-            a.steps = 3  # each step is ~15-60 s of host work; keep the arm within minutes
-        a.warmup = min(a.warmup, 1)
+        a.warmup = min(a.warmup, 1)   # each pass is ~15-60 s of host work
         run_reference_arm(a, wl, rank, world)
         return
     run_ours(a, wl, rank, world, local_rank)

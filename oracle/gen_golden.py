@@ -1,7 +1,8 @@
 """ORACLE - TEST INFRASTRUCTURE ONLY.  Generates tests/golden/*.npz by executing the REFERENCE's own
 modules (imported read-only from /root/reference, which exists only in the build container) on seeded
 synthetic inputs.  The fixtures pin oracle/hotpath.py (tests/test_oracle_golden.py) and, on the GPU box,
-the CUDA path (tests/test_gpu_parity.py).  Re-run:  python oracle/gen_golden.py
+the CUDA path (tests/test_gpu_parity.py).  It also records the state-dict inventory of the reference's full model
+(tests/golden/reference_model_inventory.json).  Re-run:  python oracle/gen_golden.py
 
 The reference has no tests/golden vectors of its own (SURVEY.md §4), so these reference-executed outputs
 are the pin.  Reference code is imported, never copied.
@@ -34,6 +35,40 @@ CASES = {
     "hotpath_v3_96x128": dict(V=3, H=96, W=128, fseed=1234, wseed=7, numdepth=192),
     "hotpath_v4_64x96": dict(V=4, H=64, W=96, fseed=99, wseed=11, numdepth=48),
 }
+
+# Arrays with many values per pixel are stored at a fixed, seeded sample of 1 / PIXEL_FRACTION of their pixels (flat
+# indices into H*W under "<key>.pixels") so that every fixture stays below 1 MB.  Depth, confidence, probability
+# logits, entropy and visibility weights are stored whole.
+SAMPLED = ("depth_values", "volume_mean", "fmt.")
+PIXEL_FRACTION = 8
+
+
+def sample_pixels(blob, seed=0):
+    out = {}
+    for k, a in blob.items():
+        if k != "meta" and any(s in k for s in SAMPLED):
+            H, W = a.shape[-2:]
+            rng = np.random.default_rng(seed)
+            idx = np.sort(rng.choice(H * W, max(1, H * W // PIXEL_FRACTION), replace=False)).astype(np.int32)
+            out[k] = np.ascontiguousarray(a.reshape(a.shape[:-2] + (H * W,))[..., idx])
+            out[k + ".pixels"] = idx
+        else:
+            out[k] = a
+    return out
+
+
+def reference_model_inventory():
+    """The reference's DINOv2MVSNet built from its shipped config: `args` and every state-dict entry as
+    [name, shape, dtype, "parameter" | "buffer"] in state-dict order (tests/test_host_cpu.py rebuilds a model of that
+    shape to check that install() keeps a reference checkpoint loadable)."""
+    from models.networks.DINOv2_mvsformer_model import DINOv2MVSNet
+    cfg = json.load(open(os.path.join(REF, "config", "mvsformer++.json")))["arch"]["args"]
+    torch.manual_seed(0)
+    model = DINOv2MVSNet(cfg)
+    params = {k for k, _ in model.named_parameters()}
+    rows = [[k, list(v.shape), str(v.dtype).replace("torch.", ""), "parameter" if k in params else "buffer"]
+            for k, v in model.state_dict().items()]
+    return {"args": cfg, "state_dict": rows}
 
 
 def make_case(c, args):
@@ -73,7 +108,7 @@ def main():
         for k in ("stage2", "stage3", "stage4"):
             blob[f"fmt.{k}.view1"] = out["features"][k][0, 1].numpy()
         blob["meta"] = np.frombuffer(json.dumps(c).encode(), dtype=np.uint8)
-        np.savez_compressed(os.path.join(out_dir, name + ".npz"), **blob)
+        np.savez_compressed(os.path.join(out_dir, name + ".npz"), **sample_pixels(blob))
         print(name, "refined_depth range", float(out["refined_depth"].min()), float(out["refined_depth"].max()),
               "stage4 conf mean", float(out["stage4"]["photometric_confidence"].mean()))
 
@@ -89,6 +124,12 @@ def main():
     np.savez_compressed(os.path.join(out_dir, "warp_seam.npz"), src=src.numpy(), src_proj=srcp.numpy(),
                         ref_proj=refp.numpy(), depth_values=dvals.numpy(), warped=warped.numpy(), mask=mask.numpy())
     print("warp_seam: fraction masked", float(mask.float().mean()))
+
+    with open(os.path.join(out_dir, "reference_model_inventory.json"), "w") as f:
+        inv = reference_model_inventory()
+        f.write('{"args": ' + json.dumps(inv["args"]) + ',\n "state_dict": [\n')
+        f.write(",\n".join("  " + json.dumps(r) for r in inv["state_dict"]) + "\n]}\n")
+    print("reference_model_inventory:", len(inv["state_dict"]), "state-dict entries")
 
 
 if __name__ == "__main__":

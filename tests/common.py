@@ -20,6 +20,13 @@ def load_golden(name):
     return d, meta
 
 
+def at_golden_pixels(gold, key, t):
+    """`t` [..., H, W] as the fixture stores `key`: whole, or at the fixed sample of pixels listed under `key`.pixels
+    (oracle/gen_golden.py keeps large arrays at a sample of their pixels)."""
+    idx = gold.get(key + ".pixels")
+    return t if idx is None else t.reshape(t.shape[:-2] + (-1,))[..., idx.long()]
+
+
 def build_case(meta, args=None):
     """Re-creates exactly the inputs oracle/gen_golden.py used (same seeds, same generators)."""
     args = args or default_args()

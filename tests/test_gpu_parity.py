@@ -11,7 +11,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from tests.common import ROOT, TMP, build_case, load_golden, max_abs, rec, rel_linf
+from tests.common import ROOT, TMP, at_golden_pixels, build_case, load_golden, max_abs, rec, rel_linf
 
 pytestmark = pytest.mark.gpu
 
@@ -473,7 +473,8 @@ def test_cascade_vs_reference_golden(cascade, s):
     name, gold, out, ora, *_ = cascade
     so = out[f"stage{s}"]
     gp = torch.softmax(gold[f"stage{s}.prob_volume_pre"], dim=0)
-    e = dict(depth_values_rel=rel_linf(so["depth_values"][0].cpu(), gold[f"stage{s}.depth_values"]),
+    key = f"stage{s}.depth_values"
+    e = dict(depth_values_rel=rel_linf(at_golden_pixels(gold, key, so["depth_values"][0].cpu()), gold[key]),
              entropy=max_abs(so["entropy"][0].cpu(), gold[f"stage{s}.entropy"]),
              vis=max_abs(so["vis_weight"][0].cpu(), gold[f"stage{s}.vis_weight"]),
              prob=max_abs(so["prob_volume"][0].cpu(), gp),
@@ -487,8 +488,9 @@ def test_cascade_final_outputs(cascade):
     name, gold, out, ora, *_ = cascade
     e = dict(refined_depth_rel=rel_linf(out["refined_depth"][0].cpu(), gold["refined_depth"]),
              confidence=max_abs(out["photometric_confidence"][0].cpu(), gold["photometric_confidence"]),
-             fmt_stage1=max_abs(out["features"]["stage1"][0].cpu(), gold["fmt.stage1"]),
-             fmt_stage4_view1=max_abs(out["features"]["stage4"][0, 1].cpu(), gold["fmt.stage4.view1"]))
+             fmt_stage1=max_abs(at_golden_pixels(gold, "fmt.stage1", out["features"]["stage1"][0].cpu()), gold["fmt.stage1"]),
+             fmt_stage4_view1=max_abs(at_golden_pixels(gold, "fmt.stage4.view1", out["features"]["stage4"][0, 1].cpu()),
+                                      gold["fmt.stage4.view1"]))
     rec(f"cascade_{name}_final", **e)
     assert e["refined_depth_rel"] < 1e-3 and e["confidence"] < 1e-4 and e["fmt_stage1"] < 2e-4
 

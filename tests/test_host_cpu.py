@@ -129,21 +129,48 @@ def test_reference_arm_reproduces_golden_fixture():
     assert torch.equal(out["photometric_confidence"][0], gold["photometric_confidence"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference repository only exists in the build container")
-def test_install_on_reference_constructed_model_keeps_the_checkpoint_contract():
-    """test.py:209-220 on the real thing: init_model -> DINOv2MVSNet(arch.args); install() swaps FMT_module / fusions for
-    this package's modules; every state-dict key and value of the model is unchanged, so a reference checkpoint loads with
-    strict=True before or after install()."""
+def _reference_shaped_model():
+    """A model with the `args` and every state-dict entry (name, shape, dtype, parameter or buffer) of the reference's
+    DINOv2MVSNet built from its shipped config, as oracle/gen_golden.py recorded them from the reference itself."""
     import json
-    import sys
-    sys.path.insert(0, "/root/reference")
-    import models.dino.layers.attention as A
-    A.FLASH_AVAILABLE = False
-    from models.networks.DINOv2_mvsformer_model import DINOv2MVSNet
+    inv = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_model_inventory.json")))
+    tree = {}
+    for name, shape, dtype, kind in inv["state_dict"]:
+        *path, leaf = name.split(".")
+        node = tree
+        for p in path:
+            node = node.setdefault(p, {})
+        node[leaf] = (shape, getattr(torch, dtype), kind)
+
+    def module(node):
+        subs = {k: module(v) for k, v in node.items() if isinstance(v, dict)}
+        if subs and all(k.isdigit() for k in subs):   # nn.ModuleList / nn.Sequential children
+            m = torch.nn.ModuleList([subs[str(i)] for i in range(len(subs))])
+        else:
+            m = torch.nn.Module()
+            for k, sub in subs.items():
+                m.add_module(k, sub)
+        for k, v in node.items():
+            if not isinstance(v, dict):
+                shape, dtype, kind = v
+                t = torch.zeros(shape, dtype=dtype)
+                if kind == "parameter":
+                    m.register_parameter(k, torch.nn.Parameter(t))
+                else:
+                    m.register_buffer(k, t)
+        return m
+
+    model = module(tree)
+    model.args = inv["args"]
+    return model
+
+
+def test_install_on_reference_constructed_model_keeps_the_checkpoint_contract():
+    """test.py:209-220: init_model -> DINOv2MVSNet(arch.args), here a model with exactly its state-dict entries;
+    install() swaps FMT_module / fusions for this package's modules; every state-dict key and value of the model is
+    unchanged, so a reference checkpoint loads with strict=True before or after install()."""
     from mvsformerplusplus_b200 import hotpath
-    cfg = json.load(open("/root/reference/config/mvsformer++.json"))["arch"]["args"]
-    torch.manual_seed(0)
-    model = DINOv2MVSNet(cfg).eval()
+    model = _reference_shaped_model().eval()
     synth.randomize_state_dict(model.FMT_module, seed=3)
     synth.randomize_state_dict(model.fusions, seed=4)
     before = {k: v.clone() for k, v in model.state_dict().items()}
