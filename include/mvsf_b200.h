@@ -81,20 +81,15 @@ int mvsf_position3d(const float* kinv_ref, const float* depth, const float* dept
 int mvsf_homo_warp(const float* src_nhwc, const float* hom, const float* depth, float* warped, uint8_t* mask, int C,
                    int D, int H, int W, mvsf_stream_t stream);
 
-/* ---- test / measurement hooks: the cost-volume passes have two organisations computing the same function - L1 gathers
+/* ---- test hooks: the cost-volume passes have two organisations computing the same function - L1 gathers
  * from global memory (warp_corr.cu, any C in 8/16/32/64) and TMA-staged shared-memory windows (warp_tile.cu, C = 8/16, even H).
  * mode 0: force the L1 organisation everywhere; 1 (default): adaptive - the window kernels of the two-gather plan where they
  * apply, and for mvsf_warp_corr_entropy_store at C = 8, D = 4 a per-call choice made ON THE DEVICE from the call's own
- * geometry (share of sampled taps that miss the pipeline kernel's predicted windows <= max_window_miss per mille ->
- * pipeline kernel, else L1 kernel; both are launched, the one not chosen returns at once); 2: force the window / pipeline
- * kernels wherever they exist.  mvsf_warp_corr_last_selection reads the most recent decision back (synchronises). */
+ * geometry (share of sampled taps that miss the pipeline kernel's predicted windows <= 60 per mille -> pipeline kernel,
+ * else L1 kernel; both are launched, the one not chosen returns at once); 2: force the window / pipeline kernels wherever
+ * they exist.  mvsf_warp_corr_last_selection reads the most recent decision back (synchronises). */
 int mvsf_warp_corr_set_tile_path(int mode);
-int mvsf_warp_corr_set_max_window_miss(int permille);
 int mvsf_warp_corr_last_selection(int* used_pipeline, int* miss_permille);
-
-/* ---- measurement hook: 1 = prefer the largest shared-memory carve-out for every kernel of the context (cudaDeviceSetCacheConfig),
- * 0 = driver default.  Used to test whether carve-out switches play a part in the two-stream deadlock (DESIGN.md 5). */
-int mvsf_set_prefer_shared_carveout(int on);
 
 /* ---- which of the two cost-volume plans to run for a stage shape: 1 = two gathers (mvsf_warp_corr_entropy, mvsf_vis_cnn,
  * mvsf_warp_corr_aggregate; no intermediate buffer), 0 = spill plan (mvsf_warp_corr_entropy_store, mvsf_vis_cnn,
@@ -106,10 +101,6 @@ int mvsf_warp_corr_plan(int C, int G, int D, int H, int W, int V, size_t spill_b
  * -> entropy [(V-1)][H][W].   The (V-1,C,D,H,W) warped volume is never written. */
 int mvsf_warp_corr_entropy(const float* feat, const float* homs, const float* depth, float* entropy, int V, int C,
                            int G, int D, int H, int W, mvsf_stream_t stream);
-/* ---- precision of the layer-2/3 activations inside the visibility CNN: 1 (default) = fp16 hi + lo (fp32-class),
- * 0 = fp16 (half the tensor-core instructions; measured against the oracle in tests/test_gpu_parity.py). */
-int mvsf_vis_cnn_set_precision(int x_lo);
-
 /* ---- W4 visibility CNN: models/cost_volume.py:37,93.  entropy [N][H][W] -> vis [N][H][W].
  * wts: packed, BN folded: w1[9][16] b1[16] w2[16 ic][9][16 oc] b2[16] w3[16 ic][9][8 oc] b3[8] w4[8] b4[1] (=3649 floats) */
 int mvsf_vis_cnn(const float* entropy, const float* wts, float* vis, int N, int H, int W, mvsf_stream_t stream);
@@ -152,11 +143,6 @@ int mvsf_costreg_tr_forward(float* volume, const float* pos, const float* wts, c
                             int layers, float softmax_scale, mvsf_stream_t stream);
 /* install-time helper: fp32 weight blob (n floats, n % 8 == 0) -> out16 = [n fp16 hi parts | n fp16 lo parts] (4n bytes) */
 int mvsf_split_weights_f16(const float* wts, void* out16, size_t n, mvsf_stream_t stream);
-
-/* ---- precision of the softmax probabilities inside the attention kernel: 0 (default) = fp16 P (one P*V product per
- * V half; the same rounded P feeds numerator and normaliser), 1 = fp16 hi + lo P (three partial products, fp32-class).
- * Both are held to the fp64 softmax attention in tests/test_gpu_parity.py; full-size cascade parity decides the default. */
-int mvsf_attention_set_precision(int p_lo);
 
 /* softmax attention of R1 alone: models/dino/layers/attention.py:141-170 (FlashAttention2.forward after the qkv linear).
  * qkv [N][3][4][16] fp32 -> out [N][64]; workspace >= (N+128)*896 bytes.  tcgen05 tensor cores, 3-term split-fp16 operands,

@@ -22,12 +22,9 @@ SIGNATURES = {
     "mvsf_position3d": ([P, P, P, I, P, I, P, I, I, I, P], I),
     "mvsf_homo_warp": ([P, P, P, P, P, I, I, I, I, P], I),
     "mvsf_warp_corr_set_tile_path": ([I], I),
-    "mvsf_warp_corr_set_max_window_miss": ([I], I),
-    "mvsf_set_prefer_shared_carveout": ([I], I),
     "mvsf_warp_corr_last_selection": ([ctypes.POINTER(I), ctypes.POINTER(I)], I),
     "mvsf_warp_corr_plan": ([I, I, I, I, I, I, Z], I),
     "mvsf_warp_corr_entropy": ([P, P, P, P, I, I, I, I, I, I, P], I),
-    "mvsf_vis_cnn_set_precision": ([I], I),
     "mvsf_vis_cnn": ([P, P, P, I, I, I, P], I),
     "mvsf_warp_corr_aggregate": ([P, P, P, P, P, I, I, I, I, I, I, P], I),
     "mvsf_warp_corr_entropy_store": ([P, P, P, P, P, I, I, I, I, I, I, P], I),
@@ -40,7 +37,6 @@ SIGNATURES = {
     "mvsf_costreg_tr_workspace_bytes": ([I, I, I, I, ctypes.POINTER(Z)], I),
     "mvsf_costreg_tr_forward": ([P, P, P, P, Z, P, P, Z, I, I, I, I, I, F, P], I),
     "mvsf_split_weights_f16": ([P, P, Z, P], I),
-    "mvsf_attention_set_precision": ([I], I),
     "mvsf_attention_forward": ([P, P, P, Z, I, F, P], I),
     "mvsf_linear_tc_forward": ([P, P, P, P, P, Z, I, I, I, I, P], I),
     "mvsf_softargmax": ([P, P, F, P, P, P, I, I, I, P], I),
@@ -48,6 +44,10 @@ SIGNATURES = {
     "mvsf_fmt_workspace_bytes": ([I, I, I, ctypes.POINTER(Z)], I),
     "mvsf_fmt_forward": ([P] * 7 + [Z] + [P] * 5 + [Z, I, I, I, P], I),
 }
+# entry points that launch no kernel: profile_calls does not time them
+NO_LAUNCH = {"mvsf_abi_version", "mvsf_launch_count", "mvsf_ktimer_enable", "mvsf_ktimer_read", "mvsf_warp_corr_plan",
+             "mvsf_warp_corr_set_tile_path", "mvsf_warp_corr_last_selection", "mvsf_costreg_unet_workspace_bytes",
+             "mvsf_costreg_unet_tc_bytes", "mvsf_costreg_tr_workspace_bytes", "mvsf_fmt_workspace_bytes"}
 
 
 def lib():
@@ -63,16 +63,6 @@ def lib():
             fn = getattr(L, name)  # AttributeError if the symbol is not exported
             fn.argtypes = argt
             fn.restype = rest
-        if os.environ.get("MVSF_ATTENTION_PLO", "0") == "1":   # A-B measurements: round-1 three-product attention
-            L.mvsf_attention_set_precision(1)
-        if os.environ.get("MVSF_VIS_XLO") in ("0", "1"):   # A-B measurements of the vis-CNN activation precision
-            L.mvsf_vis_cnn_set_precision(int(os.environ["MVSF_VIS_XLO"]))
-        if os.environ.get("MVSF_WARP_TILE", "1") in ("0", "2"):   # A-B measurements: 0 force the L1-gather kernels, 2 force the window kernels
-            L.mvsf_warp_corr_set_tile_path(int(os.environ["MVSF_WARP_TILE"]))
-        if os.environ.get("MVSF_PREFER_SHARED") in ("0", "1"):   # measurement: one shared-memory carve-out for every kernel
-            L.mvsf_set_prefer_shared_carveout(int(os.environ["MVSF_PREFER_SHARED"]))
-        if os.environ.get("MVSF_WT_MAX_MISS"):
-            L.mvsf_warp_corr_set_max_window_miss(int(os.environ["MVSF_WT_MAX_MISS"]))
         _lib = L
     return _lib
 
@@ -100,11 +90,7 @@ class profile_calls:
         L = lib()
         self._orig = {}
         for name in SIGNATURES:
-            if name.endswith("_workspace_bytes") or name in ("mvsf_abi_version", "mvsf_launch_count", "mvsf_ktimer_enable",
-                                                             "mvsf_ktimer_read", "mvsf_warp_corr_plan",
-                                                             "mvsf_warp_corr_set_tile_path", "mvsf_warp_corr_set_max_window_miss", "mvsf_set_prefer_shared_carveout",
-                                                             "mvsf_warp_corr_last_selection", "mvsf_attention_set_precision",
-                                                             "mvsf_vis_cnn_set_precision"):
+            if name in NO_LAUNCH:
                 continue
             fn = getattr(L, name)
             self._orig[name] = fn

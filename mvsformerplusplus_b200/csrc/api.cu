@@ -1,4 +1,4 @@
-// Error reporting, launch accounting and boundary layout helpers of libmvsf_b200.
+// Error reporting, launch accounting, driver entry points and boundary layout helpers of libmvsf_b200.
 #include <stdarg.h>
 #include <string.h>
 
@@ -8,6 +8,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "umma.cuh"
 
 namespace mvsf {
 static thread_local char g_err[1024] = "";
@@ -60,6 +61,17 @@ cudaEvent_t ktimer_begin(const char* name, cudaStream_t s) {
 }
 void ktimer_end(cudaEvent_t e, cudaStream_t s) { cudaEventRecord(e, s); }
 
+umma::EncodeTiledFn umma::encode_tiled_fn() {
+  static EncodeTiledFn fn = nullptr;
+  if (!fn) {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+      fn = reinterpret_cast<EncodeTiledFn>(p);
+  }
+  return fn;
+}
+
 // [N][C][HW] -> [N][HW][C] through a 32x32 shared-memory tile (coalesced on both sides)
 __global__ void transpose_chw_hwc_kernel(const float* __restrict__ src, float* __restrict__ dst, int C, int HW) {
   __shared__ float tile[32][33];
@@ -97,13 +109,6 @@ __global__ void transpose_hwc_chw_kernel(const float* __restrict__ src, float* _
 }  // namespace mvsf
 
 extern "C" {
-
-/* measurement hook (two-stream deadlock, DESIGN.md 5 / 9): ask the driver for the largest shared-memory carve-out for every
- * kernel of this context, so that an SM never has to switch carve-outs between CTAs of different kernels */
-int mvsf_set_prefer_shared_carveout(int on) {
-  MVSF_CUDA_OK(cudaDeviceSetCacheConfig(on ? cudaFuncCachePreferShared : cudaFuncCachePreferNone));
-  return MVSF_OK;
-}
 
 const char* mvsf_last_error(void) { return mvsf::g_err; }
 int mvsf_abi_version(void) { return 1; }

@@ -1,49 +1,56 @@
-// Softmax attention of the stage-1 transformer regulariser (models/module.py:507-600 -> attention.py:141-170), second
-// generation: no CTA-wide barrier in the main loop.  Included by costreg_tr.cu (uses its split_f16 / ex2f helpers).
+// Softmax attention of the stage-1 transformer regulariser (models/module.py:507-600 -> attention.py:141-170).
+// Included by costreg_tr.cu (uses its split_f16 / ex2f helpers).  No CTA-wide barrier in the main loop.
 //
 // One CTA works on TWO 128-query tiles of one head.
-//   warp 0        bulk-copy producer: K / V^T tiles (pre-tiled by qkv_tile_kernel into the canonical UMMA layouts, 4 KB
-//                 each) through two mbarrier rings; both query tiles share them
-//   warp 1        MMA issuer for both tiles, fully converged, one elected lane per tcgen05 instruction, every shared-memory
-//                 descriptor reduced to "precomputed low word + constant": the issuing warp is the critical resource
-//                 (a tcgen05.mma costs ~50 clk even stand-alone, profiles/r1_ncu_and_microbench_tcgen05.md)
-//   warps 2-9 / 10-17   softmax warps of query tile 0 / 1: two threads per query row (64 key columns each in registers),
-//                 row max exchanged through shared memory + a named barrier of the tile's 256 threads; tile 1 starts one phase late so that the two alternate between softmax and
-//                 waiting for their MMAs (ping-pong)
-// S_w(t) = Q_w K(t)^T is issued as soon as warpgroup w has pulled S_w(t-1) out of TMEM, O_w(t) = P_w(t) V(t) as soon as
-// P_w(t) is complete.  P_hi is written back to TENSOR MEMORY (tcgen05.st) and consumed as the A operand of two of the
-// three P*V products (issued as ONE MMA against [V_lo | V_hi | 1]); only P_lo travels through shared memory.  The ones
-// row of V makes the tensor core produce the softmax normaliser of the tile as well (no per-element add in the softmax
-// threads).  The partial products sit in TMEM columns that the softmax thread adds (round to nearest) while folding the
-// tile into its running output.
+//   warp 0        bulk-copy producer: the Q tiles once, then K / V^T tiles (pre-tiled by qkv_tile_kernel into the canonical
+//                 UMMA layouts, 4 KB / 12 KB each) through two mbarrier rings of NKV stages; both query tiles share them
+//   warps 1, 2    MMA issuers, one per query tile, fully converged, one elected lane per tcgen05 instruction, every
+//                 shared-memory descriptor reduced to "precomputed low word + constant": the issuing warp is the critical
+//                 resource (a tcgen05.mma costs ~50 clk even stand-alone, profiles/r1_ncu_and_microbench_tcgen05.md)
+//   warp 3        idle: keeps warp % 4 equal to the TMEM lane quarter of the softmax warps
+//   warps 4-11 / 12-19   softmax warps of query tile 0 / 1: two threads per query row (64 key columns each in registers),
+//                 row max exchanged through shared memory + a named barrier of the tile's 256 threads
+// Issuer w chains S_w(t+1) = Q_w K(t+1)^T behind "S_w(t) pulled out of TMEM" and O_w(t) = P_w(t) V(t) behind "P_w(t)
+// complete", and never waits for the other tile's events.  The softmax threads round P to fp16 (the SAME rounded P feeds
+// numerator and normaliser: an unbiased 2^-12 relative perturbation of the softmax weights) and write it back to TENSOR
+// MEMORY (tcgen05.st); it is the A operand of ONE MMA per 16 keys against [V_lo | V_hi | 1] (N = 48).  The ones row of V
+// makes the tensor core produce the softmax normaliser of the tile as well.  O_w(j-1) is folded into the running output
+// (round to nearest) after the exponentials of tile j, and the softmax warps probe their two mbarriers (S full, O full)
+// with mbarrier.test_wait a phase before they need the answer.
+//
+// Measured and removed (ms per launch at 27 648 tokens including the operand tiling; DESIGN.md §4):
+//   * P as fp16 hi + lo (P_lo through shared memory, three partial P*V products): 27 % slower, for accuracy the output
+//     cannot show (tests/test_gpu_parity.py holds the fp16 P to the fp64 softmax)
+//   * one MMA warp issuing for both tiles in a static ping-pong order: six mbarrier waits of 230-260 clk per key tile in
+//     series; two issuers + late fold + early probes took the kernel from 0.92 to 0.90 ms
+//   * fold of O(j-1) before the exponentials of tile j: 0.956 (late fold 0.940)
+//   * on top, all slower or equal (baseline 0.955): S-free / P-full signals as shared-memory counters 0.999, one mbarrier
+//     per K+V stage 0.964, pair-wise 64-thread named barriers + 4 independent max chains 1.03, one-lane polling in the
+//     softmax warps 1.11 (traced)
+//   * 2^x as a packed degree-4 polynomial on the FMA pipe for 1 / 2 / 3 of every 4 score pairs (the XU is 80 % busy):
+//     0.995 / 1.079 / 1.27 (baseline 0.940).  The 11 extra issue slots per pair cost more than the 16 XU cycles they free
+//   * in-kernel clock trace, clk per 128-key tile: softmax warp 2600 = wait S 270, TMEM -> registers 100, row max +
+//     exchange 650, 64 exponentials 1180, fold + P store 340.  A wait on an already completed mbarrier costs 120 clk on an
+//     idle SM (tools/mbar_microbench.cu) and 230-260 clk in here.  Without exponentials, row max and fold the tile still
+//     takes 2410 clk: the chain MMA -> commit -> softmax wake-up -> tcgen05.ld -> arrive -> MMA wake-up is as long as the
+//     softmax work itself.
 #pragma once
 
 namespace fa6 {
 using namespace umma;
-#ifndef MVSF_ATT_MMA2
-#define MVSF_ATT_MMA2 1   // one MMA issuer warp per query tile (warps 1, 2) instead of one warp interleaving both tiles
-#endif
-constexpr int NSOFT = 512, NCTRL = MVSF_ATT_MMA2 ? 4 : 2;   // control warps: producer, MMA issuer(s), (one idle warp keeps warp % 4 = TMEM lane quarter)
-constexpr int THREADS = 32 * NCTRL + NSOFT, NKV = 3;        // two threads per query row: 4 softmax warps per scheduler
+constexpr int NSOFT = 512, NCTRL = 4;                 // control warps: producer, two MMA issuers, one idle warp
+constexpr int THREADS = 32 * NCTRL + NSOFT, NKV = 3;  // two threads per query row: 4 softmax warps per scheduler
 constexpr uint32_t TILE = 4096;                 // one canonical 128 x 16 (Q, K) or 16 x 128 (V^T) fp16 tile
 constexpr uint32_t LBO_QK = 2048, LBO_V = 768;  // k-chunk strides: Q/K 128 rows; V^T 48 rows = V_lo dims | V_hi dims | ones row + 15 zero rows
 constexpr uint32_t V_TILE = 16 * LBO_V;         // 12 KB
-constexpr uint32_t LBO_P = 2048, P_TILE = 16 * LBO_P;
-// Q (2 tiles x hi,lo) | K ring (hi,lo) | V ring (hi,lo) | P_lo (2 warpgroups) | barriers
-constexpr uint32_t OFF_Q = 0, OFF_K = 4 * TILE, OFF_V = OFF_K + NKV * 2 * TILE, OFF_P = OFF_V + NKV * V_TILE,
-                   OFF_X = OFF_P + 2 * P_TILE, OFF_BAR = OFF_X + 4096;   // OFF_X: row-max / row-sum exchange [2 parity][2 tiles][2 halves][128]
+// Q (2 tiles x hi,lo) | K ring (hi,lo) | V ring | row-max exchange | barriers
+constexpr uint32_t OFF_Q = 0, OFF_K = 4 * TILE, OFF_V = OFF_K + NKV * 2 * TILE,
+                   OFF_X = OFF_V + NKV * V_TILE, OFF_BAR = OFF_X + 4096;   // OFF_X: row-max exchange [2 parity][2 tiles][2 halves][128]
 constexpr uint32_t SMEM = OFF_BAR + 256;
-// TMEM columns: S_w at 128 w; O_w (3 accumulators x 16) at 256 + 64 w; P_hi_w (64) at 384 + 64 w
+// TMEM columns: S_w at 128 w; O_w (P V_lo | P V_hi | sum P, 16 each) at 256 + 64 w; P_w (64 packed fp16 pairs) at 384 + 64 w
 __device__ __forceinline__ uint32_t col_s(int w) { return 128u * w; }
 __device__ __forceinline__ uint32_t col_o(int w) { return 256u + 64u * w; }
 __device__ __forceinline__ uint32_t col_p(int w) { return 384u + 64u * w; }
-__device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
 constexpr uint32_t DESC_HI = desc_hi(128);
 __device__ __forceinline__ void mma_ss(uint32_t el, uint32_t d, uint32_t alo, uint32_t blo, uint32_t idesc, uint32_t acc) {
   mma_f16_ss_lh(el, d, alo, DESC_HI, blo, DESC_HI, idesc, acc);
@@ -57,59 +64,12 @@ __device__ __forceinline__ void mma_ts(uint32_t el, uint32_t d, uint32_t ta, uin
       ::"r"(el), "r"(d), "r"(ta), "r"(blo), "r"(DESC_HI), "r"(idesc), "r"(acc)
       : "memory");
 }
-__device__ __forceinline__ void commit_e(uint32_t el, uint32_t bar) { commit_el(el, bar); }
-// Measured dead ends of round 2 (in-kernel clock trace, MVSF_ATT_TRACE; one CTA, 27 648 tokens, clk per 128-key tile):
-//   softmax warp: wait S 270, TMEM->registers 100, row max + exchange 650, 64 exponentials 1180, fold + P store 340  = 2600
-//   MMA warp:     six mbarrier waits of 240-580 clk each (a wait on an ALREADY COMPLETED mbarrier costs 120 clk on an idle SM,
-//                 tools/mbar_microbench.cu, and 230-260 clk in here), 22 MMAs issued in ~480 clk
-//   without exponentials, row max and fold (MVSF_ATT_DBG = 7) the tile still takes 2410 clk: the handshake chain
-//   MMA -> commit -> softmax wake-up -> tcgen05.ld -> arrive -> MMA-warp wake-up is as long as the softmax work itself.
-// Tried on top, all slower or equal (ms per launch incl. operand tiling, baseline 0.955): S-free / P-full signals as
-// shared-memory counters (release add per warp + polling LDS: 0.999, the release fence and the polls cost more than the
-// mbarrier), one mbarrier per K+V stage (0.964), pair-wise 64-thread named barriers + 4 independent max chains (1.03 with
-// one-lane polling), one-lane polling in the softmax warps (1.11 traced), exp2 polynomial on the FMA pipe (below).
-// 2^x for a pair of scores on the FMA pipe (packed fp32x2 instructions): round-to-nearest split x = n + f, f in [-0.5, 0.5],
-// degree-4 minimax polynomial (relative error 2.7e-6, a hundredth of the fp16 rounding P gets next), n added into the
-// exponent field.  x <= 14 by construction (running max); the clamp keeps n + 127 >= 1.
-// EXPERIMENT, off by default (MVSF_ATT_POLY_PAIRS = 0): the XU (MUFU.EX2, 16 lanes / clk / SM) is 80 % busy in this kernel,
-// so moving a share of the exponentials to the FMA pipe should pay - it does not.  Measured per launch at 27 648 tokens
-// (same accuracy, 2.5e-4 vs fp64): 0 of 4 pairs 0.940 ms, 1 of 4 0.995 ms, 2 of 4 1.079 ms, 3 of 4 1.27 ms.  The 11 extra issue
-// slots per pair (2 FMNMX + 7 packed FADD2 / FFMA2 + 2 IMAD) cost more than the 16 XU cycles they free: with 4.5 warps per
-// scheduler the softmax warps are bound by issue + dependency latency around the exponentials, not by the XU alone.
-#ifndef MVSF_ATT_FOLD_LATE
-#define MVSF_ATT_FOLD_LATE 1   // fold O(j-1) after the exponentials of tile j (0.956 -> 0.940 ms): see the softmax loop
-#endif
-#ifndef MVSF_ATT_PROBE
-#define MVSF_ATT_PROBE 1   // softmax warps probe their two mbarriers (S full, O full) a phase ahead of the point of use
-#endif
-#ifndef MVSF_ATT_TRACE
-#define MVSF_ATT_TRACE 0   // instrumented build: clock() sums per phase of the MMA warp and of four softmax warps, printed by one CTA
-#endif
-#ifndef MVSF_ATT_DBG
-#define MVSF_ATT_DBG 0   // TIMING-ONLY decomposition (results are wrong): 1 no row max / exchange / barrier, 2 no MUFU, 4 no fold, 8 one P*V MMA instead of 8, 16 one S MMA instead of 3
-#endif
-#ifndef MVSF_ATT_POLY_PAIRS
-#define MVSF_ATT_POLY_PAIRS 0   // of every 4 score pairs, how many go through the polynomial
-#endif
-__device__ __forceinline__ float2 ex2_poly2(float2 x) {
-  x.x = fmaxf(x.x, -125.0f);
-  x.y = fmaxf(x.y, -125.0f);
-  const float2 magic = make_float2(12582912.0f, 12582912.0f), neg1 = make_float2(-1.0f, -1.0f);
-  const float2 r = __fadd2_rn(x, magic);                          // low mantissa bits = n (two's complement)
-  const float2 f = __fadd2_rn(x, __ffma2_rn(r, neg1, magic));     // x - n
-  float2 p = __ffma2_rn(make_float2(0.009570101276040077f, 0.009570101276040077f), f, make_float2(0.05591785907745361f, 0.05591785907745361f));
-  p = __ffma2_rn(p, f, make_float2(0.240247443318367f, 0.240247443318367f));
-  p = __ffma2_rn(p, f, make_float2(0.6931217908859253f, 0.6931217908859253f));
-  p = __ffma2_rn(p, f, make_float2(0.9999992847442627f, 0.9999992847442627f));
-  return make_float2(__int_as_float(__float_as_int(p.x) + (__float_as_int(r.x) << 23)),
-                     __int_as_float(__float_as_int(p.y) + (__float_as_int(r.y) << 23)));
-}
 }  // namespace fa6
 
 // tiled layout: planes Qh, Ql, Kh, Kl of 4 heads x ntiles x 2048 halves (tile = [2 k-chunks][128 rows][8]) and one V plane
 // of 4 heads x ntiles x 6144 halves: V^T tile = [16 k-chunks of 8 keys][48 rows][8 keys] with rows 0-15 = dims of V_lo,
 // 16-31 = dims of V_hi, row 32 = ones (its product with P is the softmax normaliser of the tile), rows 33-47 = zero.
-// P_hi multiplies all 48 rows (N = 48), P_lo rows 16-47 (N = 32: V_hi and the ones row).  Rows / keys >= N of Q, K, V are zero.
+// P multiplies all 48 rows (N = 48).  Rows / keys >= N of Q, K, V are zero.
 __global__ void qkv_tile_kernel(const float* __restrict__ qkv, __half* __restrict__ tiled, int N, int ntiles, float qscale) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;   // (token, which, head, octet of 8 dims)
   const int total = ntiles * 128 * 3 * 4 * 2;
@@ -161,7 +121,8 @@ __global__ void qkv_tile_kernel(const float* __restrict__ qkv, __half* __restric
 //              traffic, no lo-split arithmetic in the softmax threads.  Measured against fp64 in tests/test_gpu_parity.py.
 // (Scores keep all three products Q_lo K_hi + Q_hi K_lo + Q_hi K_hi: a one-product variant measured the same 0.94 ms - the
 //  MMA warp is not the bottleneck - with 20x the error, 5.2e-3 vs fp64, and a stage-2 cascade probability error of 1.5e-4.)
-template <bool PLO>
+// Scores keep all three products Q_lo K_hi + Q_hi K_lo + Q_hi K_hi: a one-product variant measured the same 0.94 ms - the
+// MMA warp is not the bottleneck - with 20x the error, 5.2e-3 vs fp64, and a stage-2 cascade probability error of 1.5e-4.
 __global__ void __launch_bounds__(fa6::THREADS, 1)
 attention_fa_kernel(const __half* __restrict__ tiled, float* __restrict__ out, __half* __restrict__ out2, int N, int ntiles) {
   using namespace fa6;
@@ -179,8 +140,8 @@ attention_fa_kernel(const __half* __restrict__ tiled, float* __restrict__ out, _
 
   if (tid == 0) {
     mbar_init(bar_q, 1);
-    // a K / V stage is free once BOTH query tiles' products that read it are complete: one commit (MMA2: one per issuer warp)
-    for (int i = 0; i < NKV; ++i) { mbar_init(bar_kf + 8 * i, 1); mbar_init(bar_ke + 8 * i, MVSF_ATT_MMA2 ? 2 : 1); mbar_init(bar_vf + 8 * i, 1); mbar_init(bar_ve + 8 * i, MVSF_ATT_MMA2 ? 2 : 1); }
+    // a K / V stage is free once BOTH query tiles' products that read it are complete: one commit per issuer warp
+    for (int i = 0; i < NKV; ++i) { mbar_init(bar_kf + 8 * i, 1); mbar_init(bar_ke + 8 * i, 2); mbar_init(bar_vf + 8 * i, 1); mbar_init(bar_ve + 8 * i, 2); }
     for (int w = 0; w < 2; ++w) { mbar_init(bar_sf + 8 * w, 1); mbar_init(bar_sfree + 8 * w, 256); mbar_init(bar_pf + 8 * w, 256); mbar_init(bar_of + 8 * w, 1); }
     fence_barrier_init();
   }
@@ -212,126 +173,53 @@ attention_fa_kernel(const __half* __restrict__ tiled, float* __restrict__ out, _
       }
     }
   } else if (warp < NCTRL) {
-    if (MVSF_ATT_MMA2 && warp == 3) goto done;   // idle filler warp
+    if (warp == 3) goto done;   // idle filler warp
     // ------------------------------------------------------------------------------------------ MMA issuer (converged warp)
-    const uint32_t idesc_s = make_idesc_f16(128, 128), idesc_o = make_idesc_f16(128, 32), idesc_o2 = make_idesc_f16(128, 48);
+    const uint32_t idesc_s = make_idesc_f16(128, 128), idesc_o = make_idesc_f16(128, 48);
     const uint32_t el = elect_one();
     // low descriptor words of everything that does not move
     const uint32_t q_hi[2] = {desc_lo(sb + OFF_Q, LBO_QK), desc_lo(sb + OFF_Q + 2 * TILE, LBO_QK)};
     const uint32_t q_lo[2] = {desc_lo(sb + OFF_Q + TILE, LBO_QK), desc_lo(sb + OFF_Q + 3 * TILE, LBO_QK)};
-    const uint32_t p_lo[2] = {desc_lo(sb + OFF_P, LBO_P), desc_lo(sb + OFF_P + P_TILE, LBO_P)};
     const uint32_t k0 = desc_lo(sb + OFF_K, LBO_QK), v0 = desc_lo(sb + OFF_V, LBO_V);
-    // one lane polls, the warp reconverges: 32 polling lanes would steal issue slots and shared-memory bandwidth
-    auto wait1 = [&](uint32_t bar, uint32_t parity) { mbar_wait_warp(bar, parity); };
     auto issue_s = [&](int w, int t) {           // S_w(t) = Q_w K(t)^T  (K(t) has landed)
       tc_fence_after_sync();
       const uint32_t kh = k0 + (uint32_t)(t % NKV) * (2 * TILE >> 4), kl = kh + (TILE >> 4);
       const uint32_t tS = tmem_base + col_s(w);
-#if MVSF_ATT_DBG & 16
-      mma_ss(el, tS, q_hi[w], kh, idesc_s, 0u);
-#else
       mma_ss(el, tS, q_lo[w], kh, idesc_s, 0u);
       mma_ss(el, tS, q_hi[w], kl, idesc_s, 1u);
       mma_ss(el, tS, q_hi[w], kh, idesc_s, 1u);
-#endif
-      commit_e(el, bar_sf + 8 * w);
+      commit_el(el, bar_sf + 8 * w);
     };
     auto issue_pv = [&](int w, int u) {          // O_w(u) = P_w(u) V(u)  (V(u) has landed, P_w(u) is complete)
       tc_fence_after_sync();
       const uint32_t vv = v0 + (uint32_t)(u % NKV) * (V_TILE >> 4);
       const uint32_t tO = tmem_base + col_o(w), tP = tmem_base + col_p(w);
-      // two MMAs per 16 keys: P_hi (tensor memory) x [V_lo | V_hi | 1] (N = 48) -> columns [P_hi V_lo | P_hi V_hi | sum P_hi],
-      // then P_lo (shared memory) x [V_hi | 1] (N = 32) accumulated onto columns 16..47.  An MMA costs ~50 clk whatever N <= 64.
+      // one MMA per 16 keys: P (tensor memory) x [V_lo | V_hi | 1] -> columns [P V_lo | P V_hi | sum P]
 #pragma unroll
-      for (int i = 0; i < ((MVSF_ATT_DBG & 8) ? 1 : 8); ++i) {
-        mma_ts(el, tO, tP + i * 8, vv + i * (2 * LBO_V >> 4), idesc_o2, i > 0 ? 1u : 0u);
-        if (PLO) mma_ss(el, tO + 16, p_lo[w] + i * (2 * LBO_P >> 4), vv + i * (2 * LBO_V >> 4) + (256 >> 4), idesc_o, 1u);
-      }
-      commit_e(el, bar_of + 8 * w);
+      for (int i = 0; i < 8; ++i) mma_ts(el, tO, tP + i * 8, vv + i * (2 * LBO_V >> 4), idesc_o, i > 0 ? 1u : 0u);
+      commit_el(el, bar_of + 8 * w);
     };
-    // Static schedule = the order in which the events arrive when the two warpgroups alternate (warpgroup 1 starts one
-    // softmax phase after warpgroup 0): sfree0(t), pfull0(t), sfree1(t), pfull1(t), sfree0(t+1), ...
-#if MVSF_ATT_TRACE
-    uint32_t tr[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0}, tc0 = clock();
-#define ATT_TR(i) { const uint32_t c_ = clock(); tr[i] += c_ - tc0; tc0 = c_; }
-#else
-#define ATT_TR(i)
-#endif
-    auto wait_sfree = [&](int w, int t) { wait1(bar_sfree + 8 * w, (uint32_t)(t & 1)); };   // S_w(t) is in registers
-    auto wait_pf = [&](int w, int t) { wait1(bar_pf + 8 * w, (uint32_t)(t & 1)); };         // P_w(t) complete
-#if MVSF_ATT_MMA2
-    // this warp serves query tile mw alone: its chain S(t+1) <- S-free(t), P V(t) <- P-full(t) never waits for the other
-    // tile's events (a wait costs 230-260 clk even on a completed mbarrier; the single issuer went through six per tile)
-    const int mw = warp - 1;
-    wait1(bar_q, 0u);
-    wait1(bar_kf, 0u);
+    // one lane polls, the warp reconverges: 32 polling lanes would steal issue slots and shared-memory bandwidth
+    auto wait_sfree = [&](int w, int t) { mbar_wait_warp(bar_sfree + 8 * w, (uint32_t)(t & 1)); };   // S_w(t) is in registers
+    auto wait_pf = [&](int w, int t) { mbar_wait_warp(bar_pf + 8 * w, (uint32_t)(t & 1)); };         // P_w(t) complete
+    const int mw = warp - 1;   // the query tile this warp serves
+    mbar_wait_warp(bar_q, 0u);
+    mbar_wait_warp(bar_kf, 0u);
     issue_s(mw, 0);
-    commit_e(el, bar_ke);
+    commit_el(el, bar_ke);
     for (int t = 0; t < ntiles; ++t) {
       const int tn = t + 1;
       if (tn < ntiles) {
         wait_sfree(mw, t);
-        ATT_TR(0)
-        wait1(bar_kf + 8 * (tn % NKV), (uint32_t)((tn / NKV) & 1));
-        ATT_TR(1)
+        mbar_wait_warp(bar_kf + 8 * (tn % NKV), (uint32_t)((tn / NKV) & 1));
         issue_s(mw, tn);
-        commit_e(el, bar_ke + 8 * (tn % NKV));
-        ATT_TR(2)
+        commit_el(el, bar_ke + 8 * (tn % NKV));
       }
       wait_pf(mw, t);
-      ATT_TR(3)
-      wait1(bar_vf + 8 * (t % NKV), (uint32_t)((t / NKV) & 1));
-      ATT_TR(4)
+      mbar_wait_warp(bar_vf + 8 * (t % NKV), (uint32_t)((t / NKV) & 1));
       issue_pv(mw, t);
-      commit_e(el, bar_ve + 8 * (t % NKV));
-      ATT_TR(5)
+      commit_el(el, bar_ve + 8 * (t % NKV));
     }
-#else
-    wait1(bar_q, 0u);
-    wait1(bar_kf, 0u);
-    issue_s(0, 0);
-    ATT_TR(9)
-    for (int t = 0; t < ntiles; ++t) {
-      const int tn = t + 1;
-      if (tn < ntiles) {
-        wait_sfree(0, t);
-        ATT_TR(0)
-        wait1(bar_kf + 8 * (tn % NKV), (uint32_t)((tn / NKV) & 1));
-        ATT_TR(1)
-        issue_s(0, tn);
-        ATT_TR(2)
-      }
-      wait_pf(0, t);
-      ATT_TR(3)
-      wait1(bar_vf + 8 * (t % NKV), (uint32_t)((t / NKV) & 1));
-      ATT_TR(4)
-      issue_pv(0, t);
-      ATT_TR(5)
-      if (t == 0) { issue_s(1, 0); commit_e(el, bar_ke); }                        // warpgroup 1 starts here
-      if (tn < ntiles) {
-        wait_sfree(1, t);
-        ATT_TR(6)
-        issue_s(1, tn);
-        commit_e(el, bar_ke + 8 * (tn % NKV));                                    // K(t+1): both products issued
-        ATT_TR(2)
-      }
-      wait_pf(1, t);
-      ATT_TR(7)
-#if MVSF_ATT_TRACE
-      wait1(bar_q, 0u);   // a barrier that completed long ago: the fixed cost of one wait + one clock read
-      ATT_TR(8)
-#endif
-      issue_pv(1, t);
-      commit_e(el, bar_ve + 8 * (t % NKV));                                       // V(t): both products issued
-      ATT_TR(5)
-    }
-#endif
-#if MVSF_ATT_TRACE
-    if (lane == 0 && blockIdx.x == 3 && blockIdx.y == 1)
-      printf("MMA warp clk/tile: wait sfree0 %u, wait K %u, issue S (x2) %u, wait pf0 %u, wait V %u, issue PV (x2) %u, wait sfree1 %u, wait pf1 %u | total %u | a wait on a completed barrier %u\n",
-             tr[0] / ntiles, tr[1] / ntiles, tr[2] / ntiles, tr[3] / ntiles, tr[4] / ntiles, tr[5] / ntiles, tr[6] / ntiles, tr[7] / ntiles,
-             (tr[0] + tr[1] + tr[2] + tr[3] + tr[4] + tr[5] + tr[6] + tr[7]) / ntiles, tr[8] / ntiles);
-#endif
   } else {
     // ------------------------------------------------------------------------------------------ softmax warpgroups
     // 16 warps: query tile w = sw / 8, key-column half = (sw / 4) % 2, TMEM lane quarter = warp % 4.  The two threads of a
@@ -343,37 +231,26 @@ attention_fa_kernel(const __half* __restrict__ tiled, float* __restrict__ out, _
     const uint32_t lane_off = ((uint32_t)(quarter * 32)) << 16;
     const uint32_t tS = tmem_base + col_s(w) + lane_off + half * 64, tO = tmem_base + col_o(w) + lane_off + half * 8,
                    tP = tmem_base + col_p(w) + lane_off + half * 32, tOl = tmem_base + col_o(w) + lane_off + 32;
-    const uint32_t prow = sb + OFF_P + w * P_TILE + (row >> 3) * 128 + (row & 7) * 16;   // this row inside every P_lo k-chunk
     volatile float* xchg = reinterpret_cast<volatile float*>(smem + OFF_X) + w * 256;    // [parity][tile][half][128]
     float o[8];    // this thread's 8 of the 16 head dims: [8 half, 8 half + 8)
 #pragma unroll
     for (int d = 0; d < 8; ++d) o[d] = 0.f;
     float m = -1e30f, l = 0.f, corr_prev = 1.0f;
     uint32_t s_ready = 0, o_ready = 0;   // answers of the early probes (mbar_test_wait)
-    auto fold = [&](int t) {   // o = o * corr_prev + (three partial products of tile t)
+    auto fold = [&](int t) {   // o = o * corr_prev + (the two partial products of tile t)
       if (!o_ready) mbar_wait(bar_of + 8 * w, (uint32_t)(t & 1));
-#if MVSF_ATT_DBG & 4
-      return;
-#endif
       tc_fence_after_sync();
       uint32_t a0[8], a1[8], ls;
-      tmem_ld8_nowait(tO, a0);                       // P_hi V_lo
-      tmem_ld8_nowait(tO + 16, a1);                  // P_hi V_hi + P_lo V_hi
+      tmem_ld8_nowait(tO, a0);                       // P V_lo
+      tmem_ld8_nowait(tO + 16, a1);                  // P V_hi
       tmem_ld1_nowait(tOl, ls);                      // sum of the tile's P (ones row of V): the normaliser
       tmem_ld_wait();
 #pragma unroll
       for (int d = 0; d < 8; ++d) o[d] = fmaf(o[d], corr_prev, __uint_as_float(a0[d]) + __uint_as_float(a1[d]));
       l = fmaf(l, corr_prev, __uint_as_float(ls));
     };
-#if MVSF_ATT_TRACE
-    uint32_t ts[8] = {0, 0, 0, 0, 0, 0, 0, 0}, sc0 = clock();
-#define ATT_TS(i) { const uint32_t c_ = clock(); ts[i] += c_ - sc0; sc0 = c_; }
-#else
-#define ATT_TS(i)
-#endif
     for (int j = 0; j < ntiles; ++j) {
       if (!s_ready) mbar_wait(bar_sf + 8 * w, (uint32_t)(j & 1));
-      ATT_TS(0)
       tc_fence_after_sync();
       uint32_t sr[2][32];
       tmem_ld32_nowait(tS, sr[0]);
@@ -381,7 +258,6 @@ attention_fa_kernel(const __half* __restrict__ tiled, float* __restrict__ out, _
       tmem_ld_wait();
       tc_fence_before_sync();
       mbar_arrive(bar_sfree + 8 * w);          // S_w may be overwritten by the next tile's product
-      ATT_TS(1)
       if (j * 128 + 128 > N) {                 // last, partial tile only: keys >= N never win the max and get P = 0
 #pragma unroll
         for (int c = 0; c < 2; ++c)
@@ -389,101 +265,48 @@ attention_fa_kernel(const __half* __restrict__ tiled, float* __restrict__ out, _
           for (int e = 0; e < 32; ++e)
             if (j * 128 + half * 64 + c * 32 + e >= N) sr[c][e] = 0xf149f2caU;  // -1e30f
       }
-#if MVSF_ATT_DBG & 1
-      const float mx = 20.0f, corr = 1.0f;
-      m = mx;
-#else
       float pmax = -1e30f;
 #pragma unroll
       for (int c = 0; c < 2; ++c)
 #pragma unroll
         for (int e = 0; e < 32; ++e) pmax = fmaxf(pmax, __uint_as_float(sr[c][e]));
-      ATT_TS(6)
       volatile float* xj = xchg + (j & 1) * 512;
       xj[half * 128 + row] = pmax;
       if (w == 0) named_bar_sync_c<1>(256); else named_bar_sync_c<2>(256);
-      ATT_TS(7)
       const float mx = fmaxf(m, fmaxf(pmax, xj[(half ^ 1) * 128 + row]));
       const float corr = ex2f(m - mx);
       m = mx;
-#endif
-      ATT_TS(2)
-      // PLO: P_lo(j) goes to shared memory inside the loop below, so P_w(j-1) must have been consumed before it starts
-      constexpr bool FOLD_LATE = MVSF_ATT_FOLD_LATE && !PLO;
-      if (!FOLD_LATE) {
-        if (j > 0) fold(j - 1);                // also guarantees that P_w(j-1) has been consumed
-        corr_prev = corr;
-      }
-      // P is stored as fp16 hi + lo: scale it by 2^14 (largest element 16384 < 65504) so that probabilities down to 4e-12
-      // survive - without the bias every p < 3e-8 underflows to zero, a SYSTEMATIC loss of up to N * 3e-8 in the
-      // normaliser for peaked rows.  The factor cancels in O / l.
+      // P is stored as fp16: scale it by 2^14 (largest element 16384 < 65504) so that probabilities down to 4e-12 survive -
+      // without the bias every p < 3e-8 underflows to zero, a SYSTEMATIC loss of up to N * 3e-8 in the normaliser for
+      // peaked rows.  The factor cancels in O / l.
       const float mb = m - 14.0f;
       const float2 nmb2 = make_float2(-mb, -mb);
       // the answer is looked at after the exponentials: by then it has arrived, and O(j-1) is complete in all but rare cases
-      o_ready = (MVSF_ATT_PROBE && FOLD_LATE && j > 0) ? mbar_test_wait(bar_of + 8 * w, (uint32_t)((j - 1) & 1)) : 0u;
-      uint32_t pw2[2][16];
+      o_ready = j > 0 ? mbar_test_wait(bar_of + 8 * w, (uint32_t)((j - 1) & 1)) : 0u;
+      uint32_t pw[2][16];
 #pragma unroll
-      for (int c16 = 0; c16 < 2; ++c16) {      // 32 keys: one tcgen05.st of 16 packed columns, four P_lo chunks of 8 keys
-        uint32_t (&pw)[16] = pw2[c16];
+      for (int c16 = 0; c16 < 2; ++c16) {      // 32 keys: 16 packed columns of one tcgen05.st
 #pragma unroll
-        for (int c8 = 0; c8 < 4; ++c8) {
-          uint32_t pl[4];
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            // one packed fp32x2 add for the two score offsets (FADD2: half the issue slots of two FADDs)
-            const float2 xs = __fadd2_rn(make_float2(__uint_as_float(sr[c16][c8 * 8 + 2 * e]), __uint_as_float(sr[c16][c8 * 8 + 2 * e + 1])), nmb2);
-            // MVSF_ATT_POLY_PAIRS of every 4 pairs take the FMA-pipe polynomial (11 issue slots per pair, all packed or ALU)
-            // instead of two MUFU.EX2 (2 issue slots but 16 XU cycles per warp): see ex2_poly2
-            float p0, p1;
-            if (e < MVSF_ATT_POLY_PAIRS) {
-              const float2 pp = ex2_poly2(xs);
-              p0 = pp.x; p1 = pp.y;
-            } else {
-#if MVSF_ATT_DBG & 2
-              p0 = xs.x; p1 = xs.y;
-#else
-              p0 = ex2f(xs.x); p1 = ex2f(xs.y);
-#endif
-            }
-            const __half2 hh = __floats2half2_rn(p0, p1);
-            pw[c8 * 4 + e] = *reinterpret_cast<const uint32_t*>(&hh);
-            if (PLO) {
-              const float2 hf = __half22float2(hh);
-              const __half2 ll = __floats2half2_rn(p0 - hf.x, p1 - hf.y);
-              pl[e] = *reinterpret_cast<const uint32_t*>(&ll);
-            }
-          }
-          if (PLO) {
-            const uint32_t dst = prow + (half * 8 + c16 * 4 + c8) * LBO_P;
-            asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(dst), "r"(pl[0]), "r"(pl[1]), "r"(pl[2]), "r"(pl[3]) : "memory");
-          }
+        for (int e = 0; e < 16; ++e) {
+          // one packed fp32x2 add for the two score offsets (FADD2: half the issue slots of two FADDs)
+          const float2 xs = __fadd2_rn(make_float2(__uint_as_float(sr[c16][2 * e]), __uint_as_float(sr[c16][2 * e + 1])), nmb2);
+          const float p0 = ex2f(xs.x), p1 = ex2f(xs.y);
+          const __half2 hh = __floats2half2_rn(p0, p1);
+          pw[c16][e] = *reinterpret_cast<const uint32_t*>(&hh);
         }
-        if (!FOLD_LATE) tmem_st16(tP + c16 * 16, pw);
       }
-      ATT_TS(3)
       // S(j+1) was issued right after this tile's scores were pulled out of tensor memory: normally long complete
-      s_ready = (MVSF_ATT_PROBE && j + 1 < ntiles) ? mbar_test_wait(bar_sf + 8 * w, (uint32_t)((j + 1) & 1)) : 0u;
-      if (FOLD_LATE) {
-        // O_w(j-1) = P_w(j-1) V(j-1) is only needed here, a whole exponential phase after it was issued: the fold never
-        // waits for the tensor core; P_w(j) stays in registers until P_w(j-1) has been consumed
-        if (j > 0) fold(j - 1);
-        corr_prev = corr;
-        tmem_st16(tP, pw2[0]);
-        tmem_st16(tP + 16, pw2[1]);
-      }
-      ATT_TS(4)
+      s_ready = j + 1 < ntiles ? mbar_test_wait(bar_sf + 8 * w, (uint32_t)((j + 1) & 1)) : 0u;
+      // O_w(j-1) = P_w(j-1) V(j-1) is only needed here, a whole exponential phase after it was issued: the fold never waits
+      // for the tensor core; P_w(j) stays in registers until P_w(j-1) has been consumed
+      if (j > 0) fold(j - 1);
+      corr_prev = corr;
+      tmem_st16(tP, pw[0]);
+      tmem_st16(tP + 16, pw[1]);
       tmem_st_wait();
-      if (PLO) fence_proxy_async();
       tc_fence_before_sync();
       mbar_arrive(bar_pf + 8 * w);
-      ATT_TS(5)
     }
-#if MVSF_ATT_TRACE
-    if (lane == 0 && (quarter == 2) && blockIdx.x == 3 && blockIdx.y == 1)
-      printf("softmax warp %d (tile %d half %d) clk/tile: wait S %u, ld S %u, row max %u, exchange barrier %u, new max + corr %u, exps %u, fold+st %u, st wait+arrive %u | total %u\n",
-             warp, w, half, ts[0] / ntiles, ts[1] / ntiles, ts[6] / ntiles, ts[7] / ntiles, ts[2] / ntiles, ts[3] / ntiles, ts[4] / ntiles, ts[5] / ntiles,
-             (ts[0] + ts[1] + ts[2] + ts[3] + ts[4] + ts[5] + ts[6] + ts[7]) / ntiles);
-#endif
     o_ready = 0;
     fold(ntiles - 1);
     const int qt = qt0 + w;

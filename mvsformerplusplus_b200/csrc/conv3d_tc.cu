@@ -51,20 +51,6 @@ __host__ __device__ inline int npad(int cout) { return cout < 16 ? 16 : cout; }
 __host__ __device__ inline uint32_t slab_bytes(int cout) { return (uint32_t)npad(cout) * 576u; }  // 9 blocks x 2 variants x (2 x NPAD x 16 B)
 
 struct alignas(64) Maps { CUtensorMap m[4]; };   // CONV_S2: one map per (h, w) parity; otherwise m[0]
-
-__device__ __forceinline__ void expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-// TMA tile load of a 5-D box (c, w, h, d, hi/lo); out-of-range coordinates (the conv padding) are filled with zeros
-__device__ __forceinline__ void tma_load_5d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, int c3, int c4, uint32_t bar) {
-  asm volatile("cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-               ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
 }  // namespace c3
 
 // depth taps (kd, id) of output slice od
@@ -190,7 +176,7 @@ conv3d_tc_kernel(const __grid_constant__ c3::Maps maps, ConvTcArgs a, int NS, in
             const int s = g % NS;
             mbar_wait(bar_empty + 8 * s, (uint32_t)(((g / NS) & 1) ^ 1));
             const uint32_t st = sbase + s * stage_bytes, full = bar_full + 8 * s;
-            c3::expect_tx(full, (uint32_t)(KG * NSUB) * 2u * G::SUB_BYTES + b_bytes);
+            expect_tx(full, (uint32_t)(KG * NSUB) * 2u * G::SUB_BYTES + b_bytes);
             for (int og = 0; og < KG; ++og) {
               const int c = (grp * KG + og) * 8;
 #pragma unroll
@@ -199,10 +185,10 @@ conv3d_tc_kernel(const __grid_constant__ c3::Maps maps, ConvTcArgs a, int NS, in
                 if (MODE == CONV_S1) { w0 = c0w - 1; h0 = c0h - 1; }
                 else if (MODE == CONV_S2) { w0 = c0w - (sub & 1); h0 = c0h - (sub >> 1); }   // odd plane: index j <-> 2j + 1
                 else { w0 = c0w; h0 = c0h; }
-                c3::tma_load_5d(st + (uint32_t)(og * NSUB + sub) * G::PAIR, &maps.m[sub], c, w0, h0, dt.id[ds], 0, full);
+                tma_load_5d(st + (uint32_t)(og * NSUB + sub) * G::PAIR, &maps.m[sub], c, w0, h0, dt.id[ds], 0, full);
               }
             }
-            c3::bulk_load(st + a_bytes, a.wtc + (size_t)(dt.kd[ds] * ngroups + grp) * (b_bytes / 2), b_bytes, full);
+            bulk_load(st + a_bytes, a.wtc + (size_t)(dt.kd[ds] * ngroups + grp) * (b_bytes / 2), b_bytes, full);
           }
         }
       }
@@ -366,8 +352,8 @@ conv3d_col_kernel(const __grid_constant__ c3::Maps maps, ConvTcArgs a, int NS, i
     // --------------------------------------------------------------------------------------- TMA producer
     if (lane == 0) {
       if (wres) {
-        c3::expect_tx(bar_w, (uint32_t)ngroups * slab);
-        for (int grp = 0; grp < ngroups; ++grp) c3::bulk_load(wbase + grp * slab, a.wtc + (size_t)grp * (slab / 2), slab, bar_w);
+        expect_tx(bar_w, (uint32_t)ngroups * slab);
+        for (int grp = 0; grp < ngroups; ++grp) bulk_load(wbase + grp * slab, a.wtc + (size_t)grp * (slab / 2), slab, bar_w);
       }
       uint32_t g = 0;
       for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
@@ -380,7 +366,7 @@ conv3d_col_kernel(const __grid_constant__ c3::Maps maps, ConvTcArgs a, int NS, i
             const int s = g % NS;
             mbar_wait(bar_empty + 8 * s, (uint32_t)(((g / NS) & 1) ^ 1));
             const uint32_t st = ring + s * stage_bytes, full = bar_full + 8 * s;
-            c3::expect_tx(full, (uint32_t)(KG * NSUB) * 2u * G::SUB_BYTES + (wres ? 0u : slab));
+            expect_tx(full, (uint32_t)(KG * NSUB) * 2u * G::SUB_BYTES + (wres ? 0u : slab));
             for (int og = 0; og < KG; ++og) {
               const int c = (grp * KG + og) * 8;
 #pragma unroll
@@ -388,10 +374,10 @@ conv3d_col_kernel(const __grid_constant__ c3::Maps maps, ConvTcArgs a, int NS, i
                 int w0, h0;
                 if (MODE == CONV_S1) { w0 = c0w - 1; h0 = c0h - 1; }
                 else { w0 = c0w - (sub & 1); h0 = c0h - (sub >> 1); }
-                c3::tma_load_5d(st + (uint32_t)(og * NSUB + sub) * G::PAIR, &maps.m[sub], c, w0, h0, id, 0, full);
+                tma_load_5d(st + (uint32_t)(og * NSUB + sub) * G::PAIR, &maps.m[sub], c, w0, h0, id, 0, full);
               }
             }
-            if (!wres) c3::bulk_load(st + a_bytes, a.wtc + (size_t)grp * (slab / 2), slab, full);
+            if (!wres) bulk_load(st + a_bytes, a.wtc + (size_t)grp * (slab / 2), slab, full);
           }
         }
       }
@@ -611,20 +597,6 @@ int launch_merge_vec8(const __half* hi, const __half* lo, float* x, size_t n, cu
   merge_vec8_kernel<<<cdiv((long long)(n / 8), 256), 256, 0, s>>>(hi, lo, x, n / 8);
   MVSF_LAUNCH_CHECK("merge_vec8");
   return MVSF_OK;
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_tiled_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
 }
 
 // 5-D map (c, w, h, d, hi|lo) over the fp16 activation pair; sh/sw = 2 and (ph, pw) select one parity plane of (h, w)

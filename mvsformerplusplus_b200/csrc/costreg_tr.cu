@@ -136,9 +136,6 @@ __global__ void unpatch_ln_prob_kernel(const float* __restrict__ u, const float*
 }
 
 
-// 0 (default): softmax probabilities as fp16 (P_hi only); 1: fp16 hi + lo (three partial P*V products, round-1 kernel)
-static int g_attention_plo = 0;
-
 static int run_attention(const float* qkv, float* o, __half* o2, __half* tiled, int N, float scale_log2e, cudaStream_t s) {
   const int ntiles = cdiv(N, 128);
   qkv_tile_kernel<<<cdiv((long long)ntiles * 128 * 24, 256), 256, 0, s>>>(qkv, tiled, N, ntiles, scale_log2e);
@@ -146,16 +143,12 @@ static int run_attention(const float* qkv, float* o, __half* o2, __half* tiled, 
   static DeviceOnce once;
   const int dev = current_device();
   if (once.need(dev)) {
-    MVSF_CUDA_OK(cudaFuncSetAttribute(attention_fa_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fa6::SMEM));
-    MVSF_CUDA_OK(cudaFuncSetAttribute(attention_fa_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fa6::SMEM));
+    MVSF_CUDA_OK(cudaFuncSetAttribute(attention_fa_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fa6::SMEM));
     once.done(dev);
   }
   cudaEvent_t kt = ktimer_enabled() ? ktimer_begin("attention_tc", s) : nullptr;
   const dim3 grid(cdiv(ntiles, 2), 4);
-  if (g_attention_plo)
-    attention_fa_kernel<true><<<grid, fa6::THREADS, fa6::SMEM, s>>>(tiled, o, o2, N, ntiles);
-  else
-    attention_fa_kernel<false><<<grid, fa6::THREADS, fa6::SMEM, s>>>(tiled, o, o2, N, ntiles);
+  attention_fa_kernel<<<grid, fa6::THREADS, fa6::SMEM, s>>>(tiled, o, o2, N, ntiles);
   if (kt) ktimer_end(kt, s);
   MVSF_LAUNCH_CHECK("attention_tc");
   return MVSF_OK;
@@ -253,11 +246,6 @@ int mvsf_costreg_tr_forward(float* volume, const float* pos, const float* wts, c
 }
 
 /* Softmax attention alone (attention.py:141-170): qkv [N][3][4][16] fp32 -> out [N][64].  workspace >= N*768 bytes. */
-int mvsf_attention_set_precision(int p_lo) {
-  g_attention_plo = p_lo != 0;   // 0: fp16 P (default) | 1: fp16 hi+lo P (round 1)
-  return MVSF_OK;
-}
-
 int mvsf_attention_forward(const float* qkv, float* out, void* workspace, size_t workspace_bytes, int N,
                            float softmax_scale, mvsf_stream_t stream) {
   MVSF_REQUIRE(qkv && out && workspace && N > 0, "attention_forward: bad arguments");

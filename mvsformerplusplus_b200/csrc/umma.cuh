@@ -4,12 +4,14 @@
 //     i.e. 8x8 "core matrices" of 128 contiguous bytes (conflict-free for the tensor core's reads);
 //   - tcgen05.mma.cta_group::1.kind::f16 (fp16 x fp16 -> fp32 accumulators in TMEM), issued by one thread;
 //   - tcgen05.commit -> mbarrier, bounded mbarrier waits (trap instead of hanging the GPU);
+//   - bulk copies and TMA tensor-box loads into shared memory that complete on an mbarrier (expect_tx / complete_tx);
 //   - TMEM alloc/dealloc and tcgen05.ld (32 lanes x 32 bit, one accumulator row per thread).
 // Field layouts follow the PTX ISA / CUTLASS cute/arch/mma_sm100_desc.hpp (SmemDescriptor, InstrDescriptor).
 #pragma once
 #ifndef MVSF_MBAR_SPIN_LOG2
 #define MVSF_MBAR_SPIN_LOG2 26   // bounded mbarrier waits: ~1.5 s of polling before the trap
 #endif
+#include <cuda.h>
 #include <cuda_fp16.h>
 
 #include "common.cuh"
@@ -66,6 +68,27 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}" ::"r"(bar) : "memory");
 }
+// arrive and announce `bytes` of async-proxy writes that have to land before the phase completes
+__device__ __forceinline__ void expect_tx(uint32_t bar, uint32_t bytes) {
+  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+// contiguous global -> shared bulk copy (cp.async.bulk); completes `bytes` of the transaction count of `bar`
+__device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+}
+// TMA load of one 5-D box at coordinates (c0 .. c4) of `map` (a __grid_constant__ kernel parameter); coordinates outside
+// the tensor are filled with zeros
+__device__ __forceinline__ void tma_load_5d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, int c3, int c4, uint32_t bar) {
+  asm volatile("cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
+               ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
+               : "memory");
+}
+// host: the driver's cuTensorMapEncodeTiled (api.cu), nullptr when the driver does not provide it
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiledFn encode_tiled_fn();
 // named barrier among a subset of the CTA's warps (id 1..15; id 0 is __syncthreads)
 // compile-time id: a run-time id makes ptxas reserve all 16 hardware barriers (and profilers that patch the kernel then
 // cannot launch it)

@@ -23,13 +23,6 @@ namespace mvsf {
 
 using namespace umma;
 
-__device__ __forceinline__ void store_half8(__half* dst, const float (&v)[8]) {
-  __align__(16) __half h[8];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) h[e] = __float2half_rn(v[e]);
-  *reinterpret_cast<uint4*>(dst) = *reinterpret_cast<uint4*>(h);
-}
-
 namespace vc {
 constexpr int TH = 14, TW = 30;                 // output tile
 constexpr int PR = 18, PC = 34;                 // plane rows / columns (a1: all valid; a2: 16 x 32 valid, rest zero)
@@ -47,12 +40,9 @@ constexpr uint32_t OFF_A1 = 0, OFF_A2 = 4 * PLANE, OFF_B2T = 8 * PLANE, BT_LAYER
 constexpr int P_W1 = 0, P_B1 = 144, P_B2 = 160, P_B3 = 176, P_W4 = 184, P_B4 = 192;
 }  // namespace vc
 
-// XLO = true : layer-2/3 activations as fp16 hi + lo (two MMAs per tap: x_hi x [w_hi | w_lo] and x_lo x w_hi), fp32-class
-// XLO = false: activations rounded to fp16 once (x_hi x [w_hi | w_lo] only: half the MMAs - the kernel is bound by their
-//              count - and no lo planes); weights stay hi + lo.  The visibility weight is a per-pixel multiplier of the
-//              per-view correlations inside a normalised weighted mean: a relative error e on it moves the volume by
-//              e x (disagreement between views); measured vs the oracle in tests/test_gpu_parity.py.
-template <bool XLO>
+// Layer-2/3 activations stay fp16 hi + lo.  Rounding them to fp16 once (x_hi x [w_hi | w_lo] only: half the MMAs, 0.26 ms
+// less per DTU depth map) was measured and removed: 1.4e-4..4.6e-4 on the visibility weight, 1.3e-4 on the stage-4
+// probability at the full DTU size, outside the 1e-4 bar.
 __global__ void __launch_bounds__(256, 2)
 vis_cnn_kernel(const float* __restrict__ entropy, const float* __restrict__ wts, float* __restrict__ vis, int H, int W,
                int tiles_x, int tiles_y, int ntiles) {
@@ -107,10 +97,8 @@ vis_cnn_kernel(const float* __restrict__ entropy, const float* __restrict__ wts,
         // accumulator columns of M-tile ct: [32 ct, +16) = x_hi w_hi + x_lo w_hi, [32 ct + 16, +16) = x_hi w_lo
 #pragma unroll
         for (int ct = 0; ct < 4; ++ct) mma_f16_ss_lh(el, tmem_base + col + ct * 32, ah + ct * 8, a_hi, wb, b_hi, idesc32, acc);
-        if (XLO) {
 #pragma unroll
-          for (int ct = 0; ct < 4; ++ct) mma_f16_ss_lh(el, tmem_base + col + ct * 32, al + ct * 8, a_hi, wb, b_hi, idesc16, 1u);
-        }
+        for (int ct = 0; ct < 4; ++ct) mma_f16_ss_lh(el, tmem_base + col + ct * 32, al + ct * 8, a_hi, wb, b_hi, idesc16, 1u);
       }
     }
     commit_el(el, bar);
@@ -155,13 +143,8 @@ vis_cnn_kernel(const float* __restrict__ entropy, const float* __restrict__ wts,
       const float (&lo8)[8] = reinterpret_cast<const float (&)[8]>(acc[0]);
       const float (&hi8)[8] = reinterpret_cast<const float (&)[8]>(acc[8]);
       // p is a __half*: + PLANE / 2 elements = + PLANE bytes.  Planes: [hi o0 | hi o1 | lo o0 | lo o1]
-      if (XLO) {
-        split_store8(p, p + PLANE, lo8);                           // channels 0-7 : hi -> plane 0, lo -> plane 2
-        split_store8(p + PLANE / 2, p + PLANE / 2 + PLANE, hi8);   // channels 8-15: hi -> plane 1, lo -> plane 3
-      } else {
-        store_half8(p, lo8);
-        store_half8(p + PLANE / 2, hi8);
-      }
+      split_store8(p, p + PLANE, lo8);                           // channels 0-7 : hi -> plane 0, lo -> plane 2
+      split_store8(p + PLANE / 2, p + PLANE / 2 + PLANE, hi8);   // channels 8-15: hi -> plane 1, lo -> plane 3
     }
     fence_proxy_async();
     tc_fence_before_sync();
@@ -186,13 +169,8 @@ vis_cnn_kernel(const float* __restrict__ entropy, const float* __restrict__ wts,
       __half* p = reinterpret_cast<__half*>(smem + OFF_A2 + (uint32_t)(er * PC + c) * 16u);
       const float (&lo8)[8] = reinterpret_cast<const float (&)[8]>(v[0]);
       const float (&hi8)[8] = reinterpret_cast<const float (&)[8]>(v[8]);
-      if (XLO) {
-        split_store8(p, p + PLANE, lo8);
-        split_store8(p + PLANE / 2, p + PLANE / 2 + PLANE, hi8);
-      } else {
-        store_half8(p, lo8);
-        store_half8(p + PLANE / 2, hi8);
-      }
+      split_store8(p, p + PLANE, lo8);
+      split_store8(p + PLANE / 2, p + PLANE / 2 + PLANE, hi8);
     }
     fence_proxy_async();
     tc_fence_before_sync();
@@ -230,13 +208,6 @@ vis_cnn_kernel(const float* __restrict__ entropy, const float* __restrict__ wts,
 
 using namespace mvsf;
 
-static int g_vis_xlo = 1;   // 1: fp16 hi + lo activations (fp32-class), 0: fp16 activations (half the MMAs)
-
-extern "C" int mvsf_vis_cnn_set_precision(int x_lo) {
-  g_vis_xlo = x_lo != 0;
-  return MVSF_OK;
-}
-
 extern "C" int mvsf_vis_cnn(const float* entropy, const float* wts, float* vis, int N, int H, int W,
                             mvsf_stream_t stream) {
   MVSF_REQUIRE(entropy && wts && vis && N > 0 && N <= 65535 && H > 0 && W > 0, "vis_cnn: bad arguments");
@@ -244,18 +215,14 @@ extern "C" int mvsf_vis_cnn(const float* entropy, const float* wts, float* vis, 
   const int dev = current_device();
   const int num_sms = device_sm_count(dev);
   if (once.need(dev)) {
-    MVSF_CUDA_OK(cudaFuncSetAttribute(vis_cnn_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)vc::SMEM));
-    MVSF_CUDA_OK(cudaFuncSetAttribute(vis_cnn_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)vc::SMEM));
+    MVSF_CUDA_OK(cudaFuncSetAttribute(vis_cnn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)vc::SMEM));
     once.done(dev);
   }
   const int tiles_x = cdiv(W, vc::TW), tiles_y = cdiv(H, vc::TH);
   const long long ntiles = (long long)tiles_x * tiles_y * N;
   MVSF_REQUIRE(ntiles < (1ll << 30), "vis_cnn: image too large");
   const int grid = (int)(ntiles < 2 * num_sms ? ntiles : 2 * num_sms);
-  if (g_vis_xlo)
-    vis_cnn_kernel<true><<<grid, 256, vc::SMEM, (cudaStream_t)stream>>>(entropy, wts, vis, H, W, tiles_x, tiles_y, (int)ntiles);
-  else
-    vis_cnn_kernel<false><<<grid, 256, vc::SMEM, (cudaStream_t)stream>>>(entropy, wts, vis, H, W, tiles_x, tiles_y, (int)ntiles);
+  vis_cnn_kernel<<<grid, 256, vc::SMEM, (cudaStream_t)stream>>>(entropy, wts, vis, H, W, tiles_x, tiles_y, (int)ntiles);
   MVSF_LAUNCH_CHECK("vis_cnn");
   return MVSF_OK;
 }

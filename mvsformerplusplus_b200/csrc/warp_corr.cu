@@ -30,7 +30,7 @@ int warp_tile_aggregate(const float* feat, const float* homs, const float* depth
                         int D, int H, int W, cudaStream_t s);
 bool warp_stream_store_supported(const float* feat, const float* corr, int C, int G, int D, int H, int W);
 int warp_stream_entropy_store(const float* feat, const float* homs, const float* depth, float* entropy, float* corr, int V,
-                              int C, int D, int H, int W, int* select, int max_miss_permille, cudaStream_t s);
+                              int C, int D, int H, int W, int* select, cudaStream_t s);
 
 constexpr int kMaxGenericD = 512;
 
@@ -136,9 +136,8 @@ warp_corr_entropy_kernel(const float* __restrict__ feat, const float* __restrict
   const CoordConst cc = make_coord_const(W, H);
   const int y1 = p1 / W, x1 = p1 - y1 * W;
   const float fx = (float)x1, fy = (float)y1;
-  const float rx = __fadd_rn(fmaf(m.r01, fy, __fmul_rn(m.r00, fx)), m.r02);
-  const float ry = __fadd_rn(fmaf(m.r11, fy, __fmul_rn(m.r10, fx)), m.r12);
-  const float rz = __fadd_rn(fmaf(m.r21, fy, __fmul_rn(m.r20, fx)), m.r22);
+  float rx, ry, rz;
+  pixel_ray(m, fx, fy, rx, ry, rz);
   const float4 r = ldg4(feat + (size_t)p2 * C + lip * 4);
   const float* __restrict__ src = feat + (size_t)(v + 1) * HW * C + lip * 4;
   const float gscale = (float)G / (float)C;
@@ -243,9 +242,8 @@ warp_corr_aggregate_kernel(const float* __restrict__ feat, const float* __restri
     float wsum = 0.f;
     for (int v = 0; v < V - 1; ++v) {
       const Hom m = load_hom(homs + (size_t)v * 12);
-      const float rx = __fadd_rn(fmaf(m.r01, fy, __fmul_rn(m.r00, fx)), m.r02);
-      const float ry = __fadd_rn(fmaf(m.r11, fy, __fmul_rn(m.r10, fx)), m.r12);
-      const float rz = __fadd_rn(fmaf(m.r21, fy, __fmul_rn(m.r20, fx)), m.r22);
+      float rx, ry, rz;
+      pixel_ray(m, fx, fy, rx, ry, rz);
       build_taps<C>(tb, depth, m, rx, ry, rz, cc, p1, d0, D, HW, H, W, lane);
       __syncwarp();
       const float* __restrict__ src = feat + (size_t)(v + 1) * HW * C + lip * 4;
@@ -313,9 +311,8 @@ __global__ void homo_warp_kernel(const float* __restrict__ src, const float* __r
   int y = p / W, x = p - y * W;
   const Hom m = load_hom(hom);
   const float fx = (float)x, fy = (float)y;
-  const float rx = __fadd_rn(fmaf(m.r01, fy, __fmul_rn(m.r00, fx)), m.r02);
-  const float ry = __fadd_rn(fmaf(m.r11, fy, __fmul_rn(m.r10, fx)), m.r12);
-  const float rz = __fadd_rn(fmaf(m.r21, fy, __fmul_rn(m.r20, fx)), m.r22);
+  float rx, ry, rz;
+  pixel_ray(m, fx, fy, rx, ry, rz);
   const float half_w = (float)(W - 1) * 0.5f, half_h = (float)(H - 1) * 0.5f;
   float ix, iy, z;
   warp_coord(rx, ry, rz, m, __ldg(depth + (size_t)d * HW + p), half_w, half_h, (float)(W - 1), (float)(H - 1), ix, iy, z);
@@ -395,8 +392,7 @@ using namespace mvsf;
 
 // test hook: 0 forces the L1-gather organisation (warp_corr.cu) for every shape, 1 (default) lets C = 8 / 16 stages use
 // the TMA-staged window kernels (warp_tile.cu).  Both compute the same function; tests compare them.
-static int g_use_tile = 1;            // 0: L1-gather kernels everywhere, 1: adaptive (default), 2: window / pipeline kernels wherever they exist
-static int g_max_miss_permille = 60;  // adaptive choice: the pipeline kernel serves a call when <= this share of the sampled taps miss its window
+static int g_use_tile = 1;   // 0: L1-gather kernels everywhere, 1: adaptive (default), 2: window / pipeline kernels wherever they exist
 
 // Selection slots of the adaptive pass-A choice: 8 ints per call (decision, miss share, 3 scratch counters), a ring per device so that calls in
 // flight on different streams do not share a slot.  Allocated on the first call (like the kernels' attribute set-up).
@@ -426,11 +422,6 @@ extern "C" {
 
 int mvsf_warp_corr_set_tile_path(int enable) {
   g_use_tile = enable < 0 ? 0 : (enable > 2 ? 2 : enable);
-  return MVSF_OK;
-}
-int mvsf_warp_corr_set_max_window_miss(int permille) {
-  MVSF_REQUIRE(permille >= 0 && permille <= 1000, "warp_corr_set_max_window_miss: 0..1000");
-  g_max_miss_permille = permille;
   return MVSF_OK;
 }
 int mvsf_warp_corr_last_selection(int* used_pipeline, int* miss_permille) {
@@ -492,7 +483,7 @@ static int warp_corr_entropy_impl(const float* feat, const float* homs, const fl
     if (forced || C == 8) {
       int* select = forced ? nullptr : select_slot();
       if (forced || select) {
-        int rc = warp_stream_entropy_store(feat, homs, depth, entropy, corr, V, C, D, H, W, select, g_max_miss_permille, s);
+        int rc = warp_stream_entropy_store(feat, homs, depth, entropy, corr, V, C, D, H, W, select, s);
         if (rc) return rc;
         MVSF_LAUNCH_CHECK("warp_stream_entropy_store");
         if (forced) return MVSF_OK;

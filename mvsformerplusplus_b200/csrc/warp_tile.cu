@@ -27,27 +27,22 @@
 #include <cuda.h>
 #include <float.h>
 #include <limits.h>
-#include <stdlib.h>
 
-#include "common.cuh"
-
-#ifndef MVSF_PS_BLOCKS8
-#define MVSF_PS_BLOCKS8 2        // resident CTAs per SM of the C = 8 pipeline kernel (ring of MVSF_PS_NBUF8 windows of 32 KB each);
-                                 // measured at DTU stage 4: 2 CTAs x 3 windows 0.367 ms, 3 CTAs x 2 windows 0.444 ms
-#endif
-#ifndef MVSF_PS_NBUF8
-#define MVSF_PS_NBUF8 3
-#endif
-#ifndef MVSF_WT_PASSB_BLOCKS
-#define MVSF_WT_PASSB_BLOCKS 3   // resident CTAs per SM of the C = 8, D <= 4 aggregation kernel (3 costs ~20 spilled registers)
-#endif
+#include "umma.cuh"
 
 namespace mvsf {
 namespace wt {
+using namespace umma;
 
-constexpr int TW = 32, TH = 8, THREADS = 256;   // reference-pixel tile: one warp per tile row
-constexpr int DCH = 8;                          // hypotheses per window (register-resident tap coordinates)
+constexpr int TW = 32, THREADS = 256;   // reference-pixel tile: 32 columns, one warp per tile row
 constexpr int kMaxD = 512;
+// resident CTAs per SM of the C = 8 pipeline kernel and its ring of windows of 32 KB each; measured at DTU stage 4:
+// 2 CTAs x 3 windows 0.367 ms, 3 CTAs x 2 windows 0.444 ms
+constexpr int kPsBlocks8 = 2, kPsNbuf8 = 3;
+constexpr int kPassBBlocks8 = 3;   // resident CTAs per SM of the C = 8, D <= 4 aggregation kernel (3 costs ~20 spilled registers)
+// the pipeline kernel serves a pass-A call when at most this many of every 1000 sampled in-bound taps miss its windows
+// (DTU stage 4: 28, pipeline faster; Tanks&Temples: 287, L1-gather kernel faster; see warp_stream_select_kernel)
+constexpr int kMaxWindowMissPermille = 60;
 
 template <int C>
 struct Cfg {
@@ -60,34 +55,6 @@ struct Cfg {
   static constexpr uint32_t BYTES = (WY / 2) * P;    // 32 KB (C = 8), 64 KB (C = 16)
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-               : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  return ok != 0;
-}
-// one lane polls, the warp reconverges; bounded so that a mis-programmed pipeline traps instead of hanging the GPU
-__device__ __forceinline__ void mbar_wait_warp(uint32_t bar, uint32_t parity) {
-  if ((threadIdx.x & 31) == 0) {
-    uint32_t it = 0;
-    while (!mbar_try_wait(bar, parity))
-      if (++it > (1u << 26)) __trap();
-  }
-  __syncwarp();
-}
-__device__ __forceinline__ void tma_load_5d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, int c3, int c4, uint32_t bar) {
-  asm volatile("cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-               ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-               : "memory");
-}
 __device__ __forceinline__ float4 lds128(uint32_t addr) {
   float4 v;
   asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
@@ -107,6 +74,26 @@ struct Lane {
   bool b0, b1, b2;      // bits of (lane & 7) that are XORed into the bank-group index of a round
   uint32_t base[2];     // window base + 16-byte piece offset for rounds with i0 = 0 / 1
 };
+// Read order of a consumer lane that owns 8-channel slice `sub` of its pixel, with base[] relative to the window (the caller
+// adds the window address), and the first channel of the lane's quad A / quad B.
+template <int C>
+__device__ __forceinline__ Lane make_lane(int lane, int sub, int& chA, int& chB) {
+  Lane L;
+  if (C == 8) {
+    L.b0 = lane & 1; L.b1 = (lane >> 1) & 1; L.b2 = (lane >> 2) & 1;
+    L.base[0] = L.b0 ? 16 : 0;
+    L.base[1] = L.b0 ? 0 : 16;
+    chA = L.b0 ? 4 : 0; chB = L.b0 ? 0 : 4;
+  } else {
+    // lanes 2j, 2j+1 = the two channel halves of one pixel; bits 1-2 of the lane = tap slot inside an LDS.128 phase
+    L.b0 = false; L.b1 = (lane >> 1) & 1; L.b2 = (lane >> 2) & 1;
+    const int q0 = 2 * sub + (L.b1 ? 1 : 0), q1 = 2 * sub + (L.b1 ? 0 : 1);
+    L.base[0] = q0 * 16;
+    L.base[1] = q1 * 16;
+    chA = q0 * 4; chB = q1 * 4;
+  }
+  return L;
+}
 
 // One tap (4 corners x 8 channels of this lane) from the staged window: sA / sB receive the bilinear sample of the lane's
 // two channel quads (quad A = the one read in rounds with i0 = 0).  (lx, ly) = integer tap position relative to the window
@@ -189,6 +176,34 @@ __device__ __forceinline__ TapCoord split_coord(float ix, float iy, int W, int H
   return t;
 }
 
+// Origin (ox, oy even) of the WX x WY window centred on the bounding box [mnx, mxx] x [mny, mxy] of tap positions; (0, 0)
+// for an empty box.
+template <int C>
+__device__ __forceinline__ void window_origin(int mnx, int mxx, int mny, int mxy, int& ox, int& oy) {
+  using K = Cfg<C>;
+  ox = 0;
+  oy = 0;
+  if (mnx <= mxx) {
+    const int slack_x = K::WX - (mxx + 2 - mnx), slack_y = K::WY - (mxy + 2 - mny);
+    ox = mnx - (slack_x > 0 ? slack_x / 2 : 0);
+    oy = (mny - (slack_y > 0 ? slack_y / 2 : 0)) & ~1;
+  }
+}
+// The pipeline kernel's window for one (tile, view), predicted by a whole warp: each lane contributes the taps of its sample
+// pixel at the first and the last hypothesis.  The producer warp and warp_stream_select_kernel both call this, so the
+// selection replays the producer's windows exactly.
+template <int C>
+__device__ __forceinline__ void predict_window(const TapCoord& first, const TapCoord& last, int& ox, int& oy) {
+  int mnx = INT_MAX, mxx = INT_MIN, mny = INT_MAX, mxy = INT_MIN;
+  if (first.inb) { mnx = min(mnx, first.x0); mxx = max(mxx, first.x0); mny = min(mny, first.y0); mxy = max(mxy, first.y0); }
+  if (last.inb) { mnx = min(mnx, last.x0); mxx = max(mxx, last.x0); mny = min(mny, last.y0); mxy = max(mxy, last.y0); }
+  mnx = __reduce_min_sync(0xffffffffu, mnx);
+  mxx = __reduce_max_sync(0xffffffffu, mxx);
+  mny = __reduce_min_sync(0xffffffffu, mny);
+  mxy = __reduce_max_sync(0xffffffffu, mxy);
+  window_origin<C>(mnx, mxx, mny, mxy, ox, oy);
+}
+
 struct Shared {
   unsigned long long bar;
   int bbox[2][4];   // double-buffered {min x0, max x0, min y0, max y0} of the current window's taps
@@ -211,13 +226,7 @@ __device__ __forceinline__ void stage_window(const CUtensorMap* map, Shared& sh,
     atomicMax(&sh.bbox[slot][3], mxy);
   }
   __syncthreads();   // bbox complete; every lane has also finished reading the previous window
-  const int bx0 = sh.bbox[slot][0], bx1 = sh.bbox[slot][1], by0 = sh.bbox[slot][2], by1 = sh.bbox[slot][3];
-  if (bx0 > bx1) { ox = 0; oy = 0; }
-  else {
-    const int slack_x = K::WX - (bx1 + 2 - bx0), slack_y = K::WY - (by1 + 2 - by0);
-    ox = bx0 - (slack_x > 0 ? slack_x / 2 : 0);
-    oy = (by0 - (slack_y > 0 ? slack_y / 2 : 0)) & ~1;
-  }
+  window_origin<C>(sh.bbox[slot][0], sh.bbox[slot][1], sh.bbox[slot][2], sh.bbox[slot][3], ox, oy);
   if (threadIdx.x == 0) {
     sh.bbox[slot ^ 1][0] = INT_MAX; sh.bbox[slot ^ 1][1] = INT_MIN;   // reset the other slot for the next window
     sh.bbox[slot ^ 1][2] = INT_MAX; sh.bbox[slot ^ 1][3] = INT_MIN;
@@ -297,7 +306,7 @@ __device__ __forceinline__ void process_chunk(const CUtensorMap* map, Shared& sh
 // DCHT: hypotheses per window (4 or 8).  GENERIC (pass A only): D > DCHT, similarities parked in a per-thread array.
 // ----------------------------------------------------------------------------------------------------------------------
 template <int C, int MODE, int DCHT, bool GENERIC>
-__global__ void __launch_bounds__(THREADS, (C == 8 && (MODE == 0 || (DCHT == 4 && MVSF_WT_PASSB_BLOCKS == 3))) ? 3 : 2)
+__global__ void __launch_bounds__(THREADS, C == 8 && MODE == 0 ? 3 : (C == 8 && DCHT == 4 ? kPassBBlocks8 : 2))
 warp_tile_kernel(const __grid_constant__ CUtensorMap map, const float* __restrict__ feat, const float* __restrict__ homs,
                  const float* __restrict__ depth, const float* __restrict__ vis, float* __restrict__ out, int V, int D, int H,
                  int W, int dch) {
@@ -313,21 +322,10 @@ warp_tile_kernel(const __grid_constant__ CUtensorMap map, const float* __restric
   const bool active = (px < W) && (py < H);
   const int p = min(py, H - 1) * W + min(px, W - 1);
   const int sub = tid % K::LPX;           // which 8-channel slice of the pixel
-  Lane L;
-  int chA, chB;                            // first channel of the lane's quad A / quad B
-  if (C == 8) {
-    L.b0 = lane & 1; L.b1 = (lane >> 1) & 1; L.b2 = (lane >> 2) & 1;
-    L.base[0] = win + (L.b0 ? 16 : 0);
-    L.base[1] = win + (L.b0 ? 0 : 16);
-    chA = L.b0 ? 4 : 0; chB = L.b0 ? 0 : 4;
-  } else {
-    // lanes 2j, 2j+1 = the two channel halves of one pixel; bits 1-2 of the lane = tap slot inside an LDS.128 phase
-    L.b0 = false; L.b1 = (lane >> 1) & 1; L.b2 = (lane >> 2) & 1;
-    const int q0 = 2 * sub + (L.b1 ? 1 : 0), q1 = 2 * sub + (L.b1 ? 0 : 1);
-    L.base[0] = win + q0 * 16;
-    L.base[1] = win + q1 * 16;
-    chA = q0 * 4; chB = q1 * 4;
-  }
+  int chA, chB;
+  Lane L = make_lane<C>(lane, sub, chA, chB);
+  L.base[0] += win;
+  L.base[1] += win;
   if (tid == 0) {
     mbar_init(smem_u32(&sh.bar), 1);
     fence_barrier_init();
@@ -346,9 +344,7 @@ warp_tile_kernel(const __grid_constant__ CUtensorMap map, const float* __restric
   auto make_view = [&](int v) {
     ViewCtx<C> vc;
     vc.m = load_hom(homs + (size_t)v * 12);
-    vc.rx = __fadd_rn(fmaf(vc.m.r01, fyp, __fmul_rn(vc.m.r00, fxp)), vc.m.r02);
-    vc.ry = __fadd_rn(fmaf(vc.m.r11, fyp, __fmul_rn(vc.m.r10, fxp)), vc.m.r12);
-    vc.rz = __fadd_rn(fmaf(vc.m.r21, fyp, __fmul_rn(vc.m.r20, fxp)), vc.m.r22);
+    pixel_ray(vc.m, fxp, fyp, vc.rx, vc.ry, vc.rz);
     vc.srcA = feat + (size_t)(v + 1) * HW * C + chA;
     vc.srcB = feat + (size_t)(v + 1) * HW * C + chB;
     return vc;
@@ -459,11 +455,10 @@ struct PsShared {
 };
 
 template <int C, int D, int NBUF>
-__global__ void __launch_bounds__(PsCfg<C>::THREADS, (C == 8) ? MVSF_PS_BLOCKS8 : 1)
+__global__ void __launch_bounds__(PsCfg<C>::THREADS, (C == 8) ? kPsBlocks8 : 1)
 warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const float* __restrict__ feat,
                                  const float* __restrict__ homs, const float* __restrict__ depth, float* __restrict__ entropy,
-                                 float* __restrict__ corr, int V, int H, int W, int tiles_x, int ntiles, int dbg,
-                                 const int* __restrict__ select) {
+                                 float* __restrict__ corr, int V, int H, int W, int tiles_x, int ntiles, const int* __restrict__ select) {
   using K = Cfg<C>;
   using P = PsCfg<C>;
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -494,38 +489,24 @@ warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const 
       for (int v = 0; v < V - 1; ++v, ++j) {
         const int buf = j % NBUF;
         const Hom m = load_hom(homs + (size_t)v * 12);
-        const float rx = __fadd_rn(fmaf(m.r01, fyp, __fmul_rn(m.r00, fxp)), m.r02);
-        const float ry = __fadd_rn(fmaf(m.r11, fyp, __fmul_rn(m.r10, fxp)), m.r12);
-        const float rz = __fadd_rn(fmaf(m.r21, fyp, __fmul_rn(m.r20, fxp)), m.r22);
-        int mnx = INT_MAX, mxx = INT_MIN, mny = INT_MAX, mxy = INT_MIN;
+        float rx, ry, rz;
+        pixel_ray(m, fxp, fyp, rx, ry, rz);
+        TapCoord tc[2];
 #pragma unroll
         for (int e = 0; e < 2; ++e) {
           float ix, iy;
           warp_coord_lean(rx, ry, rz, m, e ? d_last : d_first, cc, ix, iy);
-          const TapCoord tc = split_coord(ix, iy, W, H);
-          if (tc.inb) { mnx = min(mnx, tc.x0); mxx = max(mxx, tc.x0); mny = min(mny, tc.y0); mxy = max(mxy, tc.y0); }
+          tc[e] = split_coord(ix, iy, W, H);
         }
-        mnx = __reduce_min_sync(0xffffffffu, mnx);
-        mxx = __reduce_max_sync(0xffffffffu, mxx);
-        mny = __reduce_min_sync(0xffffffffu, mny);
-        mxy = __reduce_max_sync(0xffffffffu, mxy);
-        int ox = 0, oy = 0;
-        if (mnx <= mxx) {
-          const int slack_x = K::WX - (mxx + 2 - mnx), slack_y = K::WY - (mxy + 2 - mny);
-          ox = mnx - (slack_x > 0 ? slack_x / 2 : 0);
-          oy = (mny - (slack_y > 0 ? slack_y / 2 : 0)) & ~1;
-        }
+        int ox, oy;
+        predict_window<C>(tc[0], tc[1], ox, oy);
         mbar_wait_warp(smem_u32(&sh.empty[buf]), (uint32_t)(((j / NBUF) & 1) ^ 1));   // consumers released this buffer
         if (lane == 0) {
           sh.origin[buf][0] = ox;
           sh.origin[buf][1] = oy;
           const uint32_t bar = smem_u32(&sh.full[buf]);
-          if (dbg & 1) {   // measurement only: no staging, the buffer is declared full at once
-            asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}" ::"r"(bar) : "memory");
-          } else {
-            expect_tx(bar, K::BYTES);
-            tma_load_5d(win0 + (uint32_t)buf * K::BYTES, &map, 0, 0, ox, oy >> 1, v + 1, bar);
-          }
+          expect_tx(bar, K::BYTES);
+          tma_load_5d(win0 + (uint32_t)buf * K::BYTES, &map, 0, 0, ox, oy >> 1, v + 1, bar);
         }
         __syncwarp();
       }
@@ -535,21 +516,9 @@ warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const 
 
   // -------------------------------------------------------------------------------------------------- consumer warps
   const int pix_in_cta = tid / K::LPX, sub = tid % K::LPX;
-  Lane L;
   int chA, chB;
-  uint32_t base0, base1;
-  if (C == 8) {
-    L.b0 = lane & 1; L.b1 = (lane >> 1) & 1; L.b2 = (lane >> 2) & 1;
-    base0 = (L.b0 ? 16 : 0);
-    base1 = (L.b0 ? 0 : 16);
-    chA = L.b0 ? 4 : 0; chB = L.b0 ? 0 : 4;
-  } else {
-    L.b0 = false; L.b1 = (lane >> 1) & 1; L.b2 = (lane >> 2) & 1;
-    const int q0 = 2 * sub + (L.b1 ? 1 : 0), q1 = 2 * sub + (L.b1 ? 0 : 1);
-    base0 = q0 * 16;
-    base1 = q1 * 16;
-    chA = q0 * 4; chB = q1 * 4;
-  }
+  Lane L = make_lane<C>(lane, sub, chA, chB);
+  const uint32_t base0 = L.base[0], base1 = L.base[1];   // + the address of the current window
   constexpr float inv_cpg = 8.0f / (float)C;
   int j = 0;
   for (int t = 0; t < my_tiles; ++t) {
@@ -565,11 +534,8 @@ warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const 
     for (int v = 0; v < V - 1; ++v, ++j) {
       const int buf = j % NBUF;
       const Hom m = load_hom(homs + (size_t)v * 12);
-      const float rx = __fadd_rn(fmaf(m.r01, fyp, __fmul_rn(m.r00, fxp)), m.r02);
-      const float ry = __fadd_rn(fmaf(m.r11, fyp, __fmul_rn(m.r10, fxp)), m.r12);
-      const float rz = __fadd_rn(fmaf(m.r21, fyp, __fmul_rn(m.r20, fxp)), m.r22);
-      const float* __restrict__ srcA = feat + (size_t)(v + 1) * HW * C + chA;
-      const float* __restrict__ srcB = feat + (size_t)(v + 1) * HW * C + chB;
+      float rx, ry, rz;
+      pixel_ray(m, fxp, fyp, rx, ry, rz);
       mbar_wait_warp(smem_u32(&sh.full[buf]), (uint32_t)((j / NBUF) & 1));
       const int ox = sh.origin[buf][0], oy = sh.origin[buf][1];
       L.base[0] = win0 + (uint32_t)buf * K::BYTES + base0;
@@ -585,13 +551,16 @@ warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const 
         float4 sA = make_float4(0.f, 0.f, 0.f, 0.f), sB = sA;
         const int lx = tc.x0 - ox, ly = tc.y0 - oy;
         const bool inwin = tc.inb && (unsigned)lx <= (unsigned)(K::WX - 2) && (unsigned)ly <= (unsigned)(K::WY - 2);
-        if (!(dbg & 2)) gather_window<C>(L, inwin ? lx : 0, inwin ? ly : 0, tc.fx, tc.fy, sA, sB);
+        gather_window<C>(L, inwin ? lx : 0, inwin ? ly : 0, tc.fx, tc.fy, sA, sB);
         if (!inwin) {
           sA = make_float4(0.f, 0.f, 0.f, 0.f); sB = sA;
-          if (tc.inb && !(dbg & 4)) gather_global<C>(srcA, srcB, ix, iy, W, H, sA, sB);
+          if (tc.inb) {   // rare: the source pointers are formed here so that they hold no registers in the loop
+            const float* __restrict__ src = feat + (size_t)(v + 1) * HW * C;
+            gather_global<C>(src + chA, src + chB, ix, iy, W, H, sA, sB);
+          }
         }
         // per-view group correlations exactly as the aggregation pass consumes them (cost_volume.py:78-85)
-        if (active && !(dbg & 8)) {
+        if (active) {
           float* cp = corr + (((size_t)v * D + k) * HW + p) * 8;
           if (C == 8) {
             *reinterpret_cast<float4*>(cp + chA) = make_float4(rA.x * sA.x, rA.y * sA.y, rA.z * sA.z, rA.w * sA.w);
@@ -608,9 +577,7 @@ warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const 
         mx = fmaxf(mx, s);
       }
       __syncwarp();
-      if (lane == 0) {   // this warp is done with the window
-        asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}" ::"r"(smem_u32(&sh.empty[buf])) : "memory");
-      }
+      if (lane == 0) mbar_arrive(smem_u32(&sh.empty[buf]));   // this warp is done with the window
       // softmax over D -> entropy (cost_volume.py:90-92).  Intrinsic exp / log (ex2 / lg2 based, ~1e-6 relative here: the
       // arguments are <= 0 resp. in (1e-7, 1]); the entropy feeds a CNN whose output is compared at 5e-4.
       float Z = 0.f, ent = 0.f;
@@ -630,14 +597,14 @@ warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const 
 // global gather, and with wide baselines + noisy hypotheses (Tanks&Temples, 9 source views: 287 per 1000, 1.57 vs 1.43 ms)
 // the L1-gather kernel is faster.  CTA b replays the producer's prediction for sample tile b (one warp per source view) and
 // counts, for the tile's 32 sample pixels, the hypotheses whose tap misses the window; the last CTA to finish turns the
-// totals into the decision and clears the scratch counters for the slot's next use.
+// totals into the decision (at most kMaxWindowMissPermille -> pipeline) and clears the scratch counters for the slot's next use.
 //   select[0] = 1: pipeline kernel, 0: L1 kernel;  select[1] = misses per 1000 in-bound taps (diagnostics);
 //   select[2..4] = scratch: taps, misses, finished CTAs (zero between calls).
 // Both kernels are launched behind it; the one not chosen returns at once.
 template <int C, int D>
 __global__ void __launch_bounds__(1024)
 warp_stream_select_kernel(const float* __restrict__ homs, const float* __restrict__ depth, int V, int H, int W, int tiles_x,
-                          int ntiles, int max_miss_permille, int* __restrict__ select) {
+                          int ntiles, int* __restrict__ select) {
   using K = Cfg<C>;
   using P = PsCfg<C>;
   const int lane = threadIdx.x & 31, HW = H * W;
@@ -653,28 +620,17 @@ warp_stream_select_kernel(const float* __restrict__ homs, const float* __restric
   unsigned int tot = 0u, miss = 0u;
   for (int v = threadIdx.x >> 5; v < V - 1; v += blockDim.x >> 5) {
     const Hom m = load_hom(homs + (size_t)v * 12);
-    const float rx = __fadd_rn(fmaf(m.r01, fyp, __fmul_rn(m.r00, fxp)), m.r02);
-    const float ry = __fadd_rn(fmaf(m.r11, fyp, __fmul_rn(m.r10, fxp)), m.r12);
-    const float rz = __fadd_rn(fmaf(m.r21, fyp, __fmul_rn(m.r20, fxp)), m.r22);
+    float rx, ry, rz;
+    pixel_ray(m, fxp, fyp, rx, ry, rz);
     TapCoord tc[D];
-    int mnx = INT_MAX, mxx = INT_MIN, mny = INT_MAX, mxy = INT_MIN;
 #pragma unroll
     for (int k = 0; k < D; ++k) {
       float ix, iy;
       warp_coord_lean(rx, ry, rz, m, dv[k], cc, ix, iy);
       tc[k] = split_coord(ix, iy, W, H);
-      if ((k == 0 || k == D - 1) && tc[k].inb) { mnx = min(mnx, tc[k].x0); mxx = max(mxx, tc[k].x0); mny = min(mny, tc[k].y0); mxy = max(mxy, tc[k].y0); }
     }
-    mnx = __reduce_min_sync(0xffffffffu, mnx);
-    mxx = __reduce_max_sync(0xffffffffu, mxx);
-    mny = __reduce_min_sync(0xffffffffu, mny);
-    mxy = __reduce_max_sync(0xffffffffu, mxy);
-    int ox = 0, oy = 0;
-    if (mnx <= mxx) {
-      const int slack_x = K::WX - (mxx + 2 - mnx), slack_y = K::WY - (mxy + 2 - mny);
-      ox = mnx - (slack_x > 0 ? slack_x / 2 : 0);
-      oy = (mny - (slack_y > 0 ? slack_y / 2 : 0)) & ~1;
-    }
+    int ox, oy;
+    predict_window<C>(tc[0], tc[D - 1], ox, oy);
 #pragma unroll
     for (int k = 0; k < D; ++k) {
       if (!tc[k].inb) continue;
@@ -694,27 +650,13 @@ warp_stream_select_kernel(const float* __restrict__ homs, const float* __restric
       const unsigned int t = (unsigned int)atomicExch(select + 2, 0), ms = (unsigned int)atomicExch(select + 3, 0);
       const unsigned int permille = t ? (unsigned int)(((unsigned long long)ms * 1000ull) / t) : 0u;
       select[1] = (int)permille;
-      select[0] = permille <= (unsigned int)max_miss_permille ? 1 : 0;
+      select[0] = permille <= (unsigned int)kMaxWindowMissPermille ? 1 : 0;
       atomicExch(select + 4, 0);
     }
   }
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_tiled_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
 // 5-D view (c, y&1, x, y/2, view) of the channels-last feature tensor [V][H][W][C] (H even)
 template <int C>
 static int make_window_map(CUtensorMap* m, const float* feat, int V, int H, int W) {
@@ -771,7 +713,7 @@ static int dispatch(int mode, const float* feat, const float* homs, const float*
 
 template <int C, int D, int NBUF>
 static int launch_stream_store(const float* feat, const float* homs, const float* depth, float* entropy, float* corr, int V,
-                               int H, int W, int* select, int max_miss_permille, cudaStream_t s) {
+                               int H, int W, int* select, cudaStream_t s) {
   using K = Cfg<C>;
   auto kern = warp_stream_entropy_store_kernel<C, D, NBUF>;
   static DeviceOnce once;
@@ -785,14 +727,13 @@ static int launch_stream_store(const float* feat, const float* homs, const float
   int rc = make_window_map<C>(&map, feat, V, H, W);
   if (rc) return rc;
   const int tiles_x = cdiv(W, TW), tiles_y = cdiv(H, PsCfg<C>::TROWS), ntiles = tiles_x * tiles_y;
-  const int per_sm = (C == 8) ? MVSF_PS_BLOCKS8 : 1;
+  const int per_sm = (C == 8) ? kPsBlocks8 : 1;
   const int cap = device_sm_count(dev) * per_sm;
-  static const int dbg = getenv("MVSF_WT_DEBUG") ? atoi(getenv("MVSF_WT_DEBUG")) : 0;   // measurement knobs (1: no staging, 2: no
   if (select) {
     const int nsample = ntiles < 96 ? ntiles : 96, warps = V - 1 < 32 ? V - 1 : 32;
-    warp_stream_select_kernel<C, D><<<nsample, 32 * warps, 0, s>>>(homs, depth, V, H, W, tiles_x, ntiles, max_miss_permille, select);
+    warp_stream_select_kernel<C, D><<<nsample, 32 * warps, 0, s>>>(homs, depth, V, H, W, tiles_x, ntiles, select);
   }
-  kern<<<ntiles < cap ? ntiles : cap, PsCfg<C>::THREADS, smem, s>>>(map, feat, homs, depth, entropy, corr, V, H, W, tiles_x, ntiles, dbg, select);   // window gather, 4: no fallback, 8: no store)
+  kern<<<ntiles < cap ? ntiles : cap, PsCfg<C>::THREADS, smem, s>>>(map, feat, homs, depth, entropy, corr, V, H, W, tiles_x, ntiles, select);
   return MVSF_OK;
 }
 
@@ -824,9 +765,9 @@ bool warp_stream_store_supported(const float* feat, const float* corr, int C, in
 // select != nullptr: five device ints (decision, miss share, three zeroed scratch counters); a small kernel decides from the geometry of THIS call whether the pipeline kernel runs
 // (select[0] = 1) or leaves the call to the L1-gather kernel the caller launches next (select[0] = 0)
 int warp_stream_entropy_store(const float* feat, const float* homs, const float* depth, float* entropy, float* corr, int V,
-                              int C, int D, int H, int W, int* select, int max_miss_permille, cudaStream_t s) {
-  if (C == 8) return wt::launch_stream_store<8, 4, MVSF_PS_NBUF8>(feat, homs, depth, entropy, corr, V, H, W, select, max_miss_permille, s);
-  return wt::launch_stream_store<16, 8, 3>(feat, homs, depth, entropy, corr, V, H, W, select, max_miss_permille, s);
+                              int C, int D, int H, int W, int* select, cudaStream_t s) {
+  if (C == 8) return wt::launch_stream_store<8, 4, wt::kPsNbuf8>(feat, homs, depth, entropy, corr, V, H, W, select, s);
+  return wt::launch_stream_store<16, 8, 3>(feat, homs, depth, entropy, corr, V, H, W, select, s);
 }
 
 }  // namespace mvsf
