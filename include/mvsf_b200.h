@@ -86,8 +86,8 @@ int mvsf_homo_warp(const float* src_nhwc, const float* hom, const float* depth, 
  * mode 0: force the L1 organisation everywhere; 1 (default): adaptive - the window kernels of the two-gather plan where they
  * apply, and for mvsf_warp_corr_entropy_store at C = 8, D = 4 a per-call choice made ON THE DEVICE from the call's own
  * geometry (share of sampled taps that miss the pipeline kernel's predicted windows <= 60 per mille -> pipeline kernel,
- * else L1 kernel; both are launched, the one not chosen returns at once); 2: force the window / pipeline kernels wherever
- * they exist.  mvsf_warp_corr_last_selection reads the most recent decision back (synchronises). */
+ * else L1 kernel; both are launched, the one not chosen returns at once); 2: force the pipeline kernel at C = 8, D = 4 and
+ * the window kernels elsewhere.  mvsf_warp_corr_last_selection reads the most recent decision back (synchronises). */
 int mvsf_warp_corr_set_tile_path(int mode);
 int mvsf_warp_corr_last_selection(int* used_pipeline, int* miss_permille);
 

@@ -10,7 +10,6 @@
 #include <cuda_fp16.h>
 #include <float.h>
 
-#include "linear.cuh"
 #include "linear_tc.cuh"
 #include "umma.cuh"
 
@@ -81,15 +80,6 @@ __global__ void patch_gather_kernel(const float* __restrict__ vol, __half* __res
   split_store8(row, row + 256, v);
 }
 
-__device__ __forceinline__ uint32_t pack_f16x2(float lo_elem, float hi_elem) {
-  uint32_t r;
-  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi_elem), "f"(lo_elem));
-  return r;
-}
-__device__ __forceinline__ float2 unpack_f16x2(uint32_t u) {
-  __half2 h = *reinterpret_cast<__half2*>(&u);
-  return __half22float2(h);  // .x = low half, .y = high half
-}
 __device__ __forceinline__ void split_f16(float x, __half& hi, __half& lo) {
   hi = __float2half_rn(x);
   lo = __float2half_rn(x - __half2float(hi));

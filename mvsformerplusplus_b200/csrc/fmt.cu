@@ -5,7 +5,6 @@
 // Tokens "(h w) c" of the reference are exactly channels-last pixels, so the stage-1 output is produced directly in
 // the [V][H][W][64] layout the warp kernels consume.  All source views are processed as one batch; the K/V
 // summaries of the two cross layers depend only on the reference view and are computed once.
-#include "linear.cuh"
 #include "linear_tc.cuh"
 #include "umma.cuh"
 

@@ -12,7 +12,9 @@
 //   pass B (warp_corr_aggregate): vol[g,d] = sum_v w_v * mean_{c in g} ref*warp_v / (sum_v w_v + 1e-6)
 //
 // Two passes because the visibility weight w_v is a 7x7-receptive-field CNN of the entropy map
-// (cost_volume.py:89-93); recomputing the gather is cheaper than spilling (V-1) x G x D x H x W floats.
+// (cost_volume.py:89-93).  Two plans bridge them: the spill plan (the cascade's default) has pass A also store the
+// (V-1) x G x D x H x W per-view group correlations and streams them in corr_aggregate_kernel; the recompute plan gathers
+// a second time in pass B and needs no buffer (plane sweeps, spill buffers over budget).  See mvsf_warp_corr_plan.
 #include <float.h>
 
 #include <atomic>
@@ -30,7 +32,7 @@ int warp_tile_aggregate(const float* feat, const float* homs, const float* depth
                         int D, int H, int W, cudaStream_t s);
 bool warp_stream_store_supported(const float* feat, const float* corr, int C, int G, int D, int H, int W);
 int warp_stream_entropy_store(const float* feat, const float* homs, const float* depth, float* entropy, float* corr, int V,
-                              int C, int D, int H, int W, int* select, cudaStream_t s);
+                              int H, int W, int* select, cudaStream_t s);
 
 constexpr int kMaxGenericD = 512;
 
@@ -329,30 +331,29 @@ __global__ void homo_warp_kernel(const float* __restrict__ src, const float* __r
 }
 
 template <int C>
-static int launch_entropy(const float* feat, const float* homs, const float* depth, float* entropy, float* corr, int V, int G,
-                          int D, int H, int W, cudaStream_t s, const int* skip_if = nullptr) {
+static void launch_entropy(const float* feat, const float* homs, const float* depth, float* entropy, float* corr, int V, int G,
+                           int D, int H, int W, cudaStream_t s) {
   constexpr int P = WC<C>::P;
   dim3 grid(cdiv((long long)H * W, 8 * P), V - 1);
-  if (skip_if) {   // adaptive launch (may find nothing to do): a capped, grid-strided grid
-    const int cap = device_sm_count(current_device()) * 16;
-    if ((int)grid.x > cap) grid.x = cap;
-    if (corr && D == WC<C>::DCH) {
-      warp_corr_entropy_kernel<C, false, C / 8, true><<<grid, 256, 0, s>>>(feat, homs, depth, entropy, corr, G, D, H, W, skip_if);
-      return 0;
-    }
-    return -1;   // only the spill plan's fixed-D instance is launched this way
-  }
   if (corr) {   // G == 8 (checked by the caller)
     if (D == WC<C>::DCH)
-      warp_corr_entropy_kernel<C, false, C / 8><<<grid, 256, 0, s>>>(feat, homs, depth, entropy, corr, G, D, H, W, skip_if);
+      warp_corr_entropy_kernel<C, false, C / 8><<<grid, 256, 0, s>>>(feat, homs, depth, entropy, corr, G, D, H, W, nullptr);
     else
-      warp_corr_entropy_kernel<C, true, C / 8><<<grid, 256, 0, s>>>(feat, homs, depth, entropy, corr, G, D, H, W, skip_if);
+      warp_corr_entropy_kernel<C, true, C / 8><<<grid, 256, 0, s>>>(feat, homs, depth, entropy, corr, G, D, H, W, nullptr);
   } else if (D == WC<C>::DCH) {
-    warp_corr_entropy_kernel<C, false, 0><<<grid, 256, 0, s>>>(feat, homs, depth, entropy, nullptr, G, D, H, W, skip_if);
+    warp_corr_entropy_kernel<C, false, 0><<<grid, 256, 0, s>>>(feat, homs, depth, entropy, nullptr, G, D, H, W, nullptr);
   } else {
-    warp_corr_entropy_kernel<C, true, 0><<<grid, 256, 0, s>>>(feat, homs, depth, entropy, nullptr, G, D, H, W, skip_if);
+    warp_corr_entropy_kernel<C, true, 0><<<grid, 256, 0, s>>>(feat, homs, depth, entropy, nullptr, G, D, H, W, nullptr);
   }
-  return 0;
+}
+// The spill plan at C = 8, D = 4 behind the selection kernel, which may have left it nothing to do (skip_if set): a capped,
+// grid-strided grid.
+static void launch_entropy_adaptive(const float* feat, const float* homs, const float* depth, float* entropy, float* corr,
+                                    int V, int G, int D, int H, int W, cudaStream_t s, const int* skip_if) {
+  constexpr int P = WC<8>::P;
+  const int blocks = cdiv((long long)H * W, 8 * P), cap = device_sm_count(current_device()) * 16;
+  dim3 grid(blocks < cap ? blocks : cap, V - 1);
+  warp_corr_entropy_kernel<8, false, 1, true><<<grid, 256, 0, s>>>(feat, homs, depth, entropy, corr, G, D, H, W, skip_if);
 }
 
 // volume[d][p][g] = sum_v vis[v][p] * corr[v][d][p][g] / (sum_v vis[v][p] + 1e-6)   (cost_volume.py:95-101), G = 8
@@ -476,22 +477,18 @@ static int warp_corr_entropy_impl(const float* feat, const float* homs, const fl
   cudaStream_t s = (cudaStream_t)stream;
   if (corr && g_use_tile && warp_stream_store_supported(feat, corr, C, G, D, H, W)) {
     // finest stage of the cascade (C = 8, D = 4): persistent TMA producer / consumer pipeline kernel, as long as the taps of
-    // this call fit its windows (decided on the device, per call: see warp_stream_select_kernel).  The C = 16, D = 8
-    // instance is not faster than the L1 kernel on either workload (DTU 0.345 vs 0.336 ms, T&T 1.88 vs 0.94 ms) and only
-    // runs when forced (mvsf_warp_corr_set_tile_path(2)).
+    // this call fit its windows (decided on the device, per call: see warp_stream_select_kernel)
     const bool forced = g_use_tile == 2;
-    if (forced || C == 8) {
-      int* select = forced ? nullptr : select_slot();
-      if (forced || select) {
-        int rc = warp_stream_entropy_store(feat, homs, depth, entropy, corr, V, C, D, H, W, select, s);
-        if (rc) return rc;
-        MVSF_LAUNCH_CHECK("warp_stream_entropy_store");
-        if (forced) return MVSF_OK;
-        count_launch();   // the selection kernel
-        launch_entropy<8>(feat, homs, depth, entropy, corr, V, G, D, H, W, s, select);   // returns at once unless select[0] == 0
-        MVSF_LAUNCH_CHECK("warp_corr_entropy");
-        return MVSF_OK;
-      }
+    int* select = forced ? nullptr : select_slot();
+    if (forced || select) {
+      int rc = warp_stream_entropy_store(feat, homs, depth, entropy, corr, V, H, W, select, s);
+      if (rc) return rc;
+      MVSF_LAUNCH_CHECK("warp_stream_entropy_store");
+      if (forced) return MVSF_OK;
+      count_launch();   // the selection kernel
+      launch_entropy_adaptive(feat, homs, depth, entropy, corr, V, G, D, H, W, s, select);   // returns at once unless select[0] == 0
+      MVSF_LAUNCH_CHECK("warp_corr_entropy");
+      return MVSF_OK;
     }
   }
   if (!corr && g_use_tile && warp_tile_supported(feat, C, G, D, H, W)) {

@@ -430,7 +430,8 @@ warp_tile_kernel(const __grid_constant__ CUtensorMap map, const float* __restric
 }
 
 // ======================================================================================================================
-// Pass A of the SPILL plan for the fine stages, as a persistent producer / consumer pipeline (the cascade's default path):
+// Pass A of the SPILL plan for the finest stage (C = 8, D = 4), as a persistent producer / consumer pipeline (the
+// cascade's default path):
 //   out: entropy[v][pixel]  and  corr[v][d][pixel][8]   (then vis CNN, then corr_aggregate streams corr).
 // One producer warp runs ahead of eight consumer warps through a ring of NBUF window buffers:
 //   producer, per (tile, view): wait empty[buf] -> predict the window origin from 32 sample pixels of the tile (first and last
@@ -441,10 +442,9 @@ warp_tile_kernel(const __grid_constant__ CUtensorMap map, const float* __restric
 // No CTA-wide barrier, no bounding-box reduction and no staging latency on the consumers' path (the first window kernels
 // above pay all three per (view, chunk) and measured 0.37 ms at DTU stage 4; the L1-gather pass A 0.51 ms).
 // ======================================================================================================================
-template <int C>
 struct PsCfg {
-  static constexpr int NCONS = 256 * Cfg<C>::LPX;   // consumer threads: an 8 x 32 pixel tile, LPX lanes per pixel
-  static constexpr int THREADS = NCONS + 32;        // + the producer warp
+  static constexpr int NCONS = 256;           // consumer threads: an 8 x 32 pixel tile, one lane per pixel
+  static constexpr int THREADS = NCONS + 32;  // + the producer warp
   static constexpr int TROWS = 8;
 };
 
@@ -455,12 +455,13 @@ struct PsShared {
 };
 
 template <int C, int D, int NBUF>
-__global__ void __launch_bounds__(PsCfg<C>::THREADS, (C == 8) ? kPsBlocks8 : 1)
+__global__ void __launch_bounds__(PsCfg::THREADS, kPsBlocks8)
 warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const float* __restrict__ feat,
                                  const float* __restrict__ homs, const float* __restrict__ depth, float* __restrict__ entropy,
                                  float* __restrict__ corr, int V, int H, int W, int tiles_x, int ntiles, const int* __restrict__ select) {
+  static_assert(C == 8, "one consumer lane per pixel owns all 8 channels");
   using K = Cfg<C>;
-  using P = PsCfg<C>;
+  using P = PsCfg;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ PsShared<NBUF> sh;
   if (select && *select == 0) return;   // warp_stream_select_kernel chose the L1-gather kernel for this call (launched next)
@@ -515,15 +516,13 @@ warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const 
   }
 
   // -------------------------------------------------------------------------------------------------- consumer warps
-  const int pix_in_cta = tid / K::LPX, sub = tid % K::LPX;
   int chA, chB;
-  Lane L = make_lane<C>(lane, sub, chA, chB);
+  Lane L = make_lane<C>(lane, 0, chA, chB);
   const uint32_t base0 = L.base[0], base1 = L.base[1];   // + the address of the current window
-  constexpr float inv_cpg = 8.0f / (float)C;
   int j = 0;
   for (int t = 0; t < my_tiles; ++t) {
     const int tile = (int)blockIdx.x + t * (int)gridDim.x;
-    const int px = (tile % tiles_x) * TW + (pix_in_cta % TW), py = (tile / tiles_x) * P::TROWS + (pix_in_cta / TW);
+    const int px = (tile % tiles_x) * TW + (tid % TW), py = (tile / tiles_x) * P::TROWS + (tid / TW);
     const bool active = (px < W) && (py < H);
     const int p = min(py, H - 1) * W + min(px, W - 1);
     const float fxp = (float)min(px, W - 1), fyp = (float)min(py, H - 1);
@@ -559,20 +558,13 @@ warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const 
             gather_global<C>(src + chA, src + chB, ix, iy, W, H, sA, sB);
           }
         }
-        // per-view group correlations exactly as the aggregation pass consumes them (cost_volume.py:78-85)
+        // per-view group correlations exactly as the aggregation pass consumes them (cost_volume.py:78-85); channels == groups
         if (active) {
           float* cp = corr + (((size_t)v * D + k) * HW + p) * 8;
-          if (C == 8) {
-            *reinterpret_cast<float4*>(cp + chA) = make_float4(rA.x * sA.x, rA.y * sA.y, rA.z * sA.z, rA.w * sA.w);
-            *reinterpret_cast<float4*>(cp + chB) = make_float4(rB.x * sB.x, rB.y * sB.y, rB.z * sB.z, rB.w * sB.w);
-          } else {
-            *reinterpret_cast<float2*>(cp + chA / 2) = make_float2(fmaf(rA.y, sA.y, rA.x * sA.x) * inv_cpg, fmaf(rA.w, sA.w, rA.z * sA.z) * inv_cpg);
-            *reinterpret_cast<float2*>(cp + chB / 2) = make_float2(fmaf(rB.y, sB.y, rB.x * sB.x) * inv_cpg, fmaf(rB.w, sB.w, rB.z * sB.z) * inv_cpg);
-          }
+          *reinterpret_cast<float4*>(cp + chA) = make_float4(rA.x * sA.x, rA.y * sA.y, rA.z * sA.z, rA.w * sA.w);
+          *reinterpret_cast<float4*>(cp + chB) = make_float4(rB.x * sB.x, rB.y * sB.y, rB.z * sB.z, rB.w * sB.w);
         }
-        float s = dot4(rA, sA) + dot4(rB, sB);
-        if (K::LPX == 2) s += __shfl_xor_sync(0xffffffffu, s, 1);
-        s *= inv_cpg;
+        const float s = dot4(rA, sA) + dot4(rB, sB);   // sum over the 8 one-channel groups
         sims[k] = s;
         mx = fmaxf(mx, s);
       }
@@ -586,7 +578,7 @@ warp_stream_entropy_store_kernel(const __grid_constant__ CUtensorMap map, const 
       const float rZ = __fdiv_rn(1.0f, Z);
 #pragma unroll
       for (int k = 0; k < D; ++k) { const float pr = sims[k] * rZ; ent -= pr * __logf(pr + 1e-7f); }
-      if (active && sub == 0) entropy[(size_t)v * HW + p] = ent;
+      if (active) entropy[(size_t)v * HW + p] = ent;
     }
   }
 }
@@ -606,7 +598,7 @@ __global__ void __launch_bounds__(1024)
 warp_stream_select_kernel(const float* __restrict__ homs, const float* __restrict__ depth, int V, int H, int W, int tiles_x,
                           int ntiles, int* __restrict__ select) {
   using K = Cfg<C>;
-  using P = PsCfg<C>;
+  using P = PsCfg;
   const int lane = threadIdx.x & 31, HW = H * W;
   const CoordConst cc = make_coord_const(W, H);
   const int sr = (lane >> 3) * 2 + 1, sc = (lane & 7) * 4 + 1;   // the producer's sample pixels
@@ -726,14 +718,13 @@ static int launch_stream_store(const float* feat, const float* homs, const float
   CUtensorMap map;
   int rc = make_window_map<C>(&map, feat, V, H, W);
   if (rc) return rc;
-  const int tiles_x = cdiv(W, TW), tiles_y = cdiv(H, PsCfg<C>::TROWS), ntiles = tiles_x * tiles_y;
-  const int per_sm = (C == 8) ? kPsBlocks8 : 1;
-  const int cap = device_sm_count(dev) * per_sm;
+  const int tiles_x = cdiv(W, TW), tiles_y = cdiv(H, PsCfg::TROWS), ntiles = tiles_x * tiles_y;
+  const int cap = device_sm_count(dev) * kPsBlocks8;
   if (select) {
     const int nsample = ntiles < 96 ? ntiles : 96, warps = V - 1 < 32 ? V - 1 : 32;
     warp_stream_select_kernel<C, D><<<nsample, 32 * warps, 0, s>>>(homs, depth, V, H, W, tiles_x, ntiles, select);
   }
-  kern<<<ntiles < cap ? ntiles : cap, PsCfg<C>::THREADS, smem, s>>>(map, feat, homs, depth, entropy, corr, V, H, W, tiles_x, ntiles, select);
+  kern<<<ntiles < cap ? ntiles : cap, PsCfg::THREADS, smem, s>>>(map, feat, homs, depth, entropy, corr, V, H, W, tiles_x, ntiles, select);
   return MVSF_OK;
 }
 
@@ -758,16 +749,15 @@ int warp_tile_aggregate(const float* feat, const float* homs, const float* depth
                 : wt::dispatch<16>(1, feat, homs, depth, vis, volume, V, D, H, W, s);
 }
 
-// pass A of the spill plan (entropy + per-view group correlations) for the shapes the pipeline kernel is built for
+// pass A of the spill plan (entropy + per-view group correlations) for the shape the pipeline kernel is built for
 bool warp_stream_store_supported(const float* feat, const float* corr, int C, int G, int D, int H, int W) {
-  return warp_tile_supported(feat, C, G, D, H, W) && ((C == 8 && D == 4) || (C == 16 && D == 8)) && ((uintptr_t)corr & 15) == 0;
+  return warp_tile_supported(feat, C, G, D, H, W) && C == 8 && D == 4 && ((uintptr_t)corr & 15) == 0;
 }
 // select != nullptr: five device ints (decision, miss share, three zeroed scratch counters); a small kernel decides from the geometry of THIS call whether the pipeline kernel runs
 // (select[0] = 1) or leaves the call to the L1-gather kernel the caller launches next (select[0] = 0)
 int warp_stream_entropy_store(const float* feat, const float* homs, const float* depth, float* entropy, float* corr, int V,
-                              int C, int D, int H, int W, int* select, cudaStream_t s) {
-  if (C == 8) return wt::launch_stream_store<8, 4, wt::kPsNbuf8>(feat, homs, depth, entropy, corr, V, H, W, select, s);
-  return wt::launch_stream_store<16, 8, 3>(feat, homs, depth, entropy, corr, V, H, W, select, s);
+                              int H, int W, int* select, cudaStream_t s) {
+  return wt::launch_stream_store<8, 4, wt::kPsNbuf8>(feat, homs, depth, entropy, corr, V, H, W, select, s);
 }
 
 }  // namespace mvsf

@@ -216,9 +216,9 @@ def test_cost_volume_kernels(dev, L, C, D, H, W, V, th, jit):
         ent_t, vis_t, vol_t = run_two_gathers()
         e_tile = dict(tile_vs_l1_entropy=max_abs(ent_t.cpu(), ent.cpu()), tile_vs_l1_volume=max_abs(vol_t.cpu(), vol_s.cpu()))
         assert e_tile["tile_vs_l1_entropy"] < 2e-5 and e_tile["tile_vs_l1_volume"] < 1e-5 * vol_scale, e_tile
-        # ... and the spill plan: forced through the persistent TMA pipeline kernel where it exists (C = 8, D = 4 and C = 16,
-        # D = 8; mode 2), then as hotpath.py runs it (mode 1: at C = 8, D = 4 the device picks pipeline or L1 kernel per call)
-        for mode in (2, 1):
+        # ... and the spill plan: forced through the persistent TMA pipeline kernel where it exists (C = 8, D = 4; mode 2),
+        # then as hotpath.py runs it (mode 1: at C = 8, D = 4 the device picks pipeline or L1 kernel per call)
+        for mode in ((2, 1) if (C, D) == (8, 4) else (1,)):
             ck(L.mvsf_warp_corr_set_tile_path(mode), "set_tile_path")
             try:
                 ent_p = torch.empty(V - 1, H, W, device=dev)
